@@ -71,7 +71,25 @@ def parse():
                          "'features' = per-level tensors with F2 only ([F2|gx|gy] derived on the device); 'concat' = per-level tensors incl. the 3C tensor")
     ap.add_argument("--precision", default="auto", choices=["auto", "fp32", "tf32x1", "tf32x2", "tf32x3", "levelwise"],
                     help="contraction path of the build kernel: auto = tensor cores (tcgen05 tf32 split-A) when K=128, else fp32 SIMT")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (R, T, W, status) to DIR/<name>.npy as float32 "
+                         "(inputs are seeded, so two builds run with the same arguments can be compared output for output)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.config != "cfg2"):
+        ap.error("--dump-outputs applies to the cfg2 solve of --impl ours")
+    return args
+
+
+def dump_outputs(out_dir, out, status):
+    """The arrays a caller of the timed step receives, as float32 .npy files (status codes are small integers: exact in float32)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    R, T, W = out
+    for name, t in (("R", R), ("T", T), ("W", W), ("status", status)):
+        if t is not None:
+            np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
 
 
 def algorithmic_bytes_per_pair_iter(N, C, K):
@@ -213,7 +231,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    reps = max(5, min(args.steps, 12))                 # bounded: a rep is one whole 640x480 pair-iteration (seconds)
+    reps = args.steps                                  # a rep is one whole 640x480 pair-iteration (seconds each)
     times, n_sample, cores = cpu_reference_sample(args.channels, args.bases, reps)
     cb, med = cpu_stats(times, n_sample, cores)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": len(times),
@@ -263,12 +281,12 @@ def run_cfg4(args):
         packed = [ops.pack_mlp([(torch.randn(dims[i], dims[i + 1], generator=g) * (2.0 / dims[i]) ** 0.5, torch.zeros(dims[i + 1])) for i in range(5)]).to(dev) for _ in LEVEL_IDS]
         ws = torch.empty(ops.lm_run_workspace_bytes(levels, _lib.PREC_AUTO), dtype=torch.uint8, device=dev)
         if joint:
-            ms = _time_ms(lambda: ops.lm_window_run(levels, iters, sc.R0, sc.T0, sc.W0[0], mlp_packed=packed, l2_regularizer_base=1000.0), max(3, args.steps))
+            ms = _time_ms(lambda: ops.lm_window_run(levels, iters, sc.R0, sc.T0, sc.W0[0], mlp_packed=packed, l2_regularizer_base=1000.0), args.steps)
             graph, ms_graph = None, None
         else:
-            ms = _time_ms(lambda: ops.lm_run(levels, iters, sc.R0, sc.T0, sc.W0, mlp_packed=packed, l2_regularizer_base=1000.0, workspace=ws), max(3, args.steps))
+            ms = _time_ms(lambda: ops.lm_run(levels, iters, sc.R0, sc.T0, sc.W0, mlp_packed=packed, l2_regularizer_base=1000.0, workspace=ws), args.steps)
             graph = ops.LMRunGraph(levels, iters, mlp_packed=packed, l2_regularizer_base=1000.0)       # the same call captured once into a CUDA graph
-            ms_graph = _time_ms(lambda: graph.solve(sc.R0, sc.T0, sc.W0), max(3, args.steps))
+            ms_graph = _time_ms(lambda: graph.solve(sc.R0, sc.T0, sc.W0), args.steps)
         N_tot = sum(l.N for l in sc.levels)
         # sparse points: no texel reuse, every point reads its own 4 taps of the 3C map
         by = nb * iters * sum((4 * l.N * (2 * C + K + 4) if npts is None else 4 * l.N * (C + 12 * C + K + 4)) + 4 * ((6 + K) ** 2 + 6 + K + C) for l in sc.levels)
@@ -278,7 +296,7 @@ def run_cfg4(args):
                     "pair_iters_per_s_cuda_graph": None if ms_graph is None else nb * len(levels) * iters / (ms_graph * 1e-3)})
         del sc, levels, graph
         torch.cuda.empty_cache()
-    print(json.dumps({"metric": METRIC, "unit": UNIT, "value": out[0]["pair_iters_per_s"], "n_gpus": 1, "higher_is_better": True, "data": "synthetic",
+    print(json.dumps({"metric": METRIC, "unit": UNIT, "value": out[0]["pair_iters_per_s"], "n_gpus": 1, "steps": args.steps, "higher_is_better": True, "data": "synthetic",
                       "config": {"workload": "cfg4: keyframe + 4 frames as nb=4 pairs, 640x480 4-level pyramid, K=128, 10 LM iters/level; dense (F2-only layout) "
                                              "and sparse N=4096 random sub-pixel points per level ([F2|gx|gy] layout, ragged tiles)", "precision": "auto"},
                       "variants": out, "roofline": {"bound": "hbm (dense) / launch+latency (sparse)", "peak": peak, "peak_kind": peak_kind, "unit": "GB/s"}}))
@@ -306,7 +324,7 @@ def run_cfg5(args):
             if name == "tensor_core" and K == 256:
                 row[name] = None                   # K = 256 runs on the SIMT path only (no tensor-core instantiation: 2 x 272 TMEM columns > 512)
                 continue
-            reps = 2 if (name == "fp32_simt" and K >= 128) else 3
+            reps = args.steps
             ms_b = _time_ms(lambda: ops.lm_build(lv[0], sc.R0, sc.T0, W0, precision=prec), reps, warm=1)
             ms_s = _time_ms(lambda: ops.lm_run(lv, iters, sc.R0, sc.T0, W0, lambda_fixed=0.05, precision=prec), reps, warm=1)
             by = nb * algorithmic_bytes_per_pair_iter(l.N, C, K)
@@ -316,7 +334,7 @@ def run_cfg5(args):
         del B, lv
         torch.cuda.empty_cache()
     best = max(r["tensor_core"]["pair_iters_per_s"] for r in sweep if r["K"] == 128 and r["tensor_core"])
-    print(json.dumps({"metric": METRIC, "unit": UNIT, "value": best, "n_gpus": 1, "higher_is_better": True, "data": "synthetic",
+    print(json.dumps({"metric": METRIC, "unit": UNIT, "value": best, "n_gpus": 1, "steps": args.steps, "higher_is_better": True, "data": "synthetic",
                       "config": {"workload": f"cfg5: K sweep at 640x480 (one dense level), nb={nb}, C={C}, 5 LM iters, fixed lambda; F2-only layout", "precision": "auto vs fp32"},
                       "sweep": sweep, "roofline": {"bound": "hbm", "peak": peak, "peak_kind": peak_kind, "unit": "GB/s",
                                                    "alg_bytes_per_pair_iter": "4*N*(2C+K+4) + 4*(P^2+P+C)", "tensor_flops_per_pair_iter": "2*N*K*(K+7)"}}))
@@ -420,6 +438,8 @@ def main():
         ms = float(tms.item())
     ms_per_step = ms / args.steps
     value = world * nb * total_iters / (ms_per_step * 1e-3)
+    if rank == 0 and args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, out, status)
 
     # ---- roofline of the dominant kernel (lm_build_kernel), per level, CUDA events on the launch stream ----
     peak, peak_kind = measured_peaks()

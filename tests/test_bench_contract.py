@@ -33,5 +33,5 @@ def test_committed_bench_line_has_every_contract_key():
 def test_bench_cli_parses():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert out.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--precision", "--layout", "--e2e-boundary", "--config", "--motion"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--precision", "--layout", "--e2e-boundary", "--config", "--motion", "--dump-outputs"):
         assert flag in out.stdout

@@ -104,28 +104,53 @@ def test_lm_build_tensorcore_matches_oracle(C, fly, n_points, grid, hw, prec):
     assert torch.equal(H, H.transpose(1, 2))
 
 
-def test_lm_run_tensorcore_vs_oracle_outputs():
+_PORTABLE_CASE = r'''
+import sys, torch
+sys.path[:0] = sys.argv[2:]
+torch.backends.mkldnn.enabled = False
+from helpers import O, scene_case, oracle_level_inputs
+sc = scene_case(nb=2, H=96, W=128, C=64, K=128, level_ids=(2, 3), seed=91, dtype=torch.float32)
+
+def oracle(dtype):
+    olv = []
+    for l in sc.levels:
+        a = oracle_level_inputs(l, dtype)
+        olv.append(O.LevelInputs(a["conv1"], a["conv2"], a["fx"], a["fy"], a["ox"], a["oy"], a["p"], a["D"], a["B"], []))
+    opts = O.IterOptions(lambda_override=torch.full((2,), 0.05, dtype=dtype))
+    return O.lm_solve(olv, 3, sc.R0.to(dtype), sc.T0.to(dtype), sc.W0.to(dtype), opts)
+
+torch.save({"levels": [{k: getattr(l, k) for k in ("conv1", "conv2", "intr", "p", "D", "B")} for l in sc.levels],
+            "R0": sc.R0, "T0": sc.T0, "W0": sc.W0, "oracle64": oracle(torch.float64), "oracle32": oracle(torch.float32)}, sys.argv[1])
+'''
+
+
+def _portable_cpu_case(tmp_dir):
+    """The scene of test_lm_run_tensorcore_vs_oracle_outputs and the oracle's float64 and float32 solves of it, computed with CPU
+    arithmetic that does not depend on the host: MKL in conditional-numerical-reproducibility mode, ATen's baseline kernels and oneDNN
+    off (each selects instruction-set-specific float32 kernels otherwise).  Both settings are read when torch loads, hence the subprocess."""
+    import os, subprocess, sys
+    here = os.path.dirname(os.path.abspath(__file__))
+    out = os.path.join(str(tmp_dir), "case.pt")
+    env = dict(os.environ, MKL_CBWR="COMPATIBLE", ATEN_CPU_CAPABILITY="default")
+    subprocess.run([sys.executable, "-c", _PORTABLE_CASE, out, here, os.path.dirname(here)], env=env, check=True)
+    return torch.load(out)
+
+
+def test_lm_run_tensorcore_vs_oracle_outputs(tmp_path):
     """Whole solve (2 levels x 3 iterations, fixed lambda, K=128) in every precision mode against the float64 oracle.
     Bar: the 1e-4 north-star tolerance on R, T, W — or, where the problem is too ill-conditioned for ANY fp32
-    implementation, twice the error of the oracle itself run in float32 (the reference's arithmetic type)."""
+    implementation, twice the error of the oracle itself run in float32 (the reference's arithmetic type).
+    The case and both oracle runs come from _portable_cpu_case: with the host's own float32 CPU kernels, the scene and
+    the float32 oracle's W error depend on the CPU the test runs on (8e-5 to 4.5e-4 across the ISA paths of one CPU)."""
     from banet_b200 import ops
-    sc = scene_case(nb=2, H=96, W=128, C=64, K=128, level_ids=(2, 3), seed=91, dtype=torch.float32)
-    levels = [ops.Level(to_cuda32(l.conv1), to_cuda32(l.conv2), to_cuda32(l.intr), to_cuda32(l.p), to_cuda32(l.D), to_cuda32(l.B)) for l in sc.levels]
-
-    def oracle(dtype):
-        olv = []
-        for l in sc.levels:
-            a = oracle_level_inputs(l, dtype)
-            olv.append(O.LevelInputs(a["conv1"], a["conv2"], a["fx"], a["fy"], a["ox"], a["oy"], a["p"], a["D"], a["B"], []))
-        opts = O.IterOptions(lambda_override=torch.full((2,), 0.05, dtype=dtype))
-        return O.lm_solve(olv, 3, sc.R0.to(dtype), sc.T0.to(dtype), sc.W0.to(dtype), opts)
-
-    oR, oT, oW = oracle(torch.float64)
-    fR, fT, fW = oracle(torch.float32)
+    case = _portable_cpu_case(tmp_path)
+    levels = [ops.Level(*[to_cuda32(l[k]) for k in ("conv1", "conv2", "intr", "p", "D", "B")]) for l in case["levels"]]
+    oR, oT, oW = case["oracle64"]
+    fR, fT, fW = case["oracle32"]
     floor = (rel_fro(fR, oR), rel_fro(fT, oT), rel_fro(fW, oW))
     print(f"oracle fp32 vs fp64 (noise floor): {floor[0]:.2e} {floor[1]:.2e} {floor[2]:.2e}")
     for prec in (0, 3, 2, 1):
-        R, T, W, status = ops.lm_run(levels, 3, to_cuda32(sc.R0), to_cuda32(sc.T0), to_cuda32(sc.W0), lambda_fixed=0.05, precision=prec)
+        R, T, W, status = ops.lm_run(levels, 3, *[to_cuda32(case[k]) for k in ("R0", "T0", "W0")], lambda_fixed=0.05, precision=prec)
         errs = (rel_fro(R, oR), rel_fro(T, oT), rel_fro(W, oW))
         print(f"prec={prec}: rel-fro R,T,W = {errs[0]:.2e} {errs[1]:.2e} {errs[2]:.2e}")
         assert status.abs().max().item() == 0
