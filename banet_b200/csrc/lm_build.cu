@@ -505,7 +505,7 @@ int lm_build_simt(const banet_level_t* lv, const BuildPlan& plan, const float* R
     prm.slot_floats = plan.slot_floats; prm.max_span = plan.max_span;
     prm.tiles_per_pair = plan.tiles_per_pair; prm.total_tiles = plan.total_tiles;
     prm.kq_i = 0; prm.kq_j = 0;
-    prm.grid_w = 0; prm.grid_h = 0; prm.tiles_x = 0; prm.tiles_y = 0; prm.band_rows = 1; prm.l2_hints = 0; prm.tap_prefetch = 0; prm.hdd_transposed = 0; prm.force_direct = 0; prm.trace = nullptr;
+    prm.grid_w = 0; prm.grid_h = 0; prm.tiles_x = 0; prm.tiles_y = 0; prm.band_rows = 1; prm.l2_hints = 0; prm.tap_prefetch = 0; prm.hdd_transposed = 0; prm.force_direct = 0;
     const bool vec4 = (lv->C % 4 == 0) && (lv->conv2_channels % 4 == 0) &&
                       ((reinterpret_cast<uintptr_t>(lv->conv1) | reinterpret_cast<uintptr_t>(lv->conv2)) % 16 == 0);
     int rc;

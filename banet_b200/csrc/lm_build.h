@@ -17,7 +17,6 @@ struct BuildParams {
     int l2_hints;                     // generation 6: 0 none, 1 read-once streams evict-first, 2 = 1 + taps evict-last
     int hdd_transposed;               // tensor-core path stores the H_dd block of a slot column-major (coalesced TMEM drains)
     int force_direct;                 // generation 7, testing: take the global-tap fallback for every tile
-    long long* trace;                 // optional debug timeline buffer (NULL in production)
 };
 
 struct BuildPlan {
@@ -35,7 +34,7 @@ int lm_build_simt(const banet_level_t* lv, const BuildPlan& plan, const float* R
 
 int launch_lm_reduce(const BuildParams& prm, int grid_build, float* H, float* g, float* rbar_sum, float* nvalid, cudaStream_t st);
 
-// tensor-core path (lm_build_tc_host.cu + lm_build_tc6.cu / lm_build_tc7.cu): K in {32,64,128}, C in {64,128}
+// tensor-core path (lm_build_tc_host.cu + lm_build_tc6.cu / lm_build_tc7.cu on lm_build_tc_roles.cuh): K in {32,64,128}, C in {64,128}
 void set_tuning(const banet_tuning_t& t);
 const banet_tuning_t& tuning();
 void lm_build_tc7_window(int* wx, int* wy);

@@ -1,54 +1,39 @@
 // lm_build_tc6.cu — tensor-core build kernel, generation 6: every phase has its own warpgroup, phases of different tiles overlap.
 //
-// Contract, slot layout and precision modes: see lm_build_tc_host.cu.  Roles (896 threads, 1 CTA / SM; register budgets by setmaxnreg,
-// 48 / 88 / 72 / 32 = 64 512 of the SM's 65 536 registers):
+// Roles, barriers and the pipeline code both generations share: lm_build_tc_roles.cuh.  What generation 6 does in them (register budgets by
+// setmaxnreg, 48 / 88 / 72 / 32 = 64 512 of the SM's 65 536 registers):
 //
-//   warpgroup 0    4 geometry warps, 16 pixels each per tile, run ahead of everybody:                              (48 regs)
-//                    b.W from the TMA-staged basis tile, warp / mask / tap offsets -> pixel records (ring of NREC)
-//   warpgroups 1-4 16 gather warps, 4 pixels each per tile: records -> 13 tap loads -> blend / accumulate -> M, q  (88 regs)
-//   warpgroup 5    4 algebra warps, 16 pixels each per tile:                                                        (72 regs)
-//                    2x7 per-pixel algebra (H_cc / g_c partials in registers), R rows (A_lo, R_lo) into smem,
-//                    then ONE elected thread issues the tile's tcgen05.mma and refills the freed basis stage by TMA
-//   warpgroup 6    4 drainer warps (one TMEM lane quadrant each): TMEM chains -> partial slots (L2 evict-last), asynchronous (32 regs)
-//   mbarriers: fullB[NST] TMA landed | recs[NREC] geometry->gather | gath[NREC] gather->algebra | recfree[NREC] algebra->geometry |
-//              rfree MMAs of the tile done (R, A_lo and the A stage reusable) | chain_done/drained[2], flushb, tmemfree issuer<->drainers |
-//              rbdump/rbfree gather<->algebra hand-over of the |diff| sums at a pair change.
-#include "common.cuh"
-#include "lm_build.h"
-#include "tc_utils.cuh"
+//   geometry warps (48 regs)  b.W; in MODE 1 they also round the basis tile to tf32 in place; tap offsets -> pixel records
+//   gather warps   (88 regs)  13 tap loads per (pixel, 4 channels) by ld.global -> blend / accumulate -> M, q
+//   algebra warps  (72 regs)  besides the shared algebra: the R rows s_n * b_n (A_lo, R_lo) into smem; L2-hinted basis TMA
+//   drainer warps  (32 regs)
+#include "lm_build_tc_roles.cuh"
 #include "tmap.h"
 #include <stdlib.h>
 
 namespace banet { namespace v6 {
-using namespace tc;
+using namespace tcb;
 
-constexpr int TILE = 64, W0 = 4, GW = 16, AW = 4, DW = 4;      // geometry | gather | algebra | drainer warps
-constexpr int THREADS = (W0 + GW + AW + DW) * 32;               // 896
-constexpr int KB = 128, NN = 160;
-constexpr int STAGE_A = 4 * TILE * 128, STAGE_R = 5 * TILE * 128;
-constexpr int REC = 16;
-constexpr int CHAIN = 8, TMEM_COLS = 512, ACCL = 320;
+__device__ __forceinline__ float hsum16(float v) {
+    v += __shfl_xor_sync(0xffffffffu, v, 8); v += __shfl_xor_sync(0xffffffffu, v, 4);
+    v += __shfl_xor_sync(0xffffffffu, v, 2); v += __shfl_xor_sync(0xffffffffu, v, 1);
+    return v;
+}
 
 template <int MODE, bool FLY> struct Smem {
-#ifndef BANET_TC6_NST
-#define BANET_TC6_NST 4
-#endif
-#ifndef BANET_TC6_NREC
-#define BANET_TC6_NREC 3
-#endif
     // basis-tile stages (TMA ring) and pixel-record buffers.  Deeper rings decouple the roles, but whatever smem the CTA takes is lost
     // to the L1 that catches the tap overlap of neighbouring pixels: measured best per mode / layout (640x480, 32 pairs):
     //   TF32X2 + [F2|gx|gy] layout: 3 stages (192 KB -> 196 KB carve-out, 60 KB L1) 7.4 ms vs 4 stages (228 KB) 8.6 ms
     //   TF32X2 + F2-only layout   : 4 stages 7.2 ms vs 3 stages 8.8 ms;  TF32X1: 4 stages 5.6 ms vs 3 stages 6.1 ms
-    static constexpr int NST = MODE == 3 ? 3 : (MODE == 2 && !FLY) ? 3 : BANET_TC6_NST;
-    static constexpr int NREC = MODE == 3 ? 2 : BANET_TC6_NREC;
+    static constexpr int NST = MODE == 3 ? 3 : (MODE == 2 && !FLY) ? 3 : 4;
+    static constexpr int NREC = MODE == 3 ? 2 : 3;
     static constexpr int off_A = 0;
     static constexpr int off_R = NST * STAGE_A;
     static constexpr int off_Alo = off_R + STAGE_R;
     static constexpr int off_Rlo = off_Alo + (MODE >= 2 ? STAGE_A : 0);
     static constexpr int off_misc = off_Rlo + (MODE == 3 ? STAGE_R : 0);
-    static constexpr int off_bar = off_misc;                           // 22 mbarriers
-    static constexpr int off_tmem = off_bar + 22 * 8;
+    static constexpr int off_bar = off_misc;                           // NBARS mbarriers
+    static constexpr int off_tmem = off_bar + NBARS * 8;
     static constexpr int off_tile = off_misc + 192;                    // [NREC][4] ints: pair index of the tile in record buffer s
     static constexpr int off_pose = off_tile + 64;                     // [W0][16] floats (private to each geometry warp)
     static constexpr int off_w = off_pose + W0 * 16 * 4;               // [W0][128] floats: W of the pair (private to each geometry warp)
@@ -60,41 +45,6 @@ template <int MODE, bool FLY> struct Smem {
     static constexpr int bytes = total + slack;
 };
 
-__device__ __forceinline__ long long gtime6() { long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
-// debug timeline (BANET_TC_TRACE_PTR): CTA 1, gather warp 0 (role 0), algebra warp 0 (role 1) and geometry warp 0 (role 2), tiles 16..47, 12 stamps each
-#ifdef BANET_TC6_TRACE_ON
-#define TC6_TRACE(role, it, slot) do { if (prm.trace && blockIdx.x == 1 && lane == 0 && (it) >= 16 && (it) < 48) \
-        prm.trace[(((role) * 32 + ((it) - 16)) * 12) + (slot)] = gtime6(); } while (0)
-#else
-#define TC6_TRACE(role, it, slot) do { } while (0)
-#endif
-template <int NT> __device__ __forceinline__ void team_bar() { asm volatile("bar.sync 2, %0;" :: "n"(NT) : "memory"); }
-__device__ __forceinline__ int reflect_i(int i, int n) { i = i < 0 ? -i : (i >= n ? 2 * n - 2 - i : i); return i < 0 ? 0 : i; }
-__device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
-__device__ __forceinline__ float hsum16(float v) {
-    v += __shfl_xor_sync(0xffffffffu, v, 8); v += __shfl_xor_sync(0xffffffffu, v, 4);
-    v += __shfl_xor_sync(0xffffffffu, v, 2); v += __shfl_xor_sync(0xffffffffu, v, 1);
-    return v;
-}
-struct TileCoord { int b, n0, cnt, tx0, ty0; };
-__device__ __forceinline__ TileCoord tile_coord(const BuildParams& prm, long long tl) {
-    TileCoord tc;
-    const unsigned t = (unsigned)tl, tpp = (unsigned)prm.tiles_per_pair;
-    tc.b = (int)(t / tpp);
-    const int r = (int)(t - (unsigned)tc.b * tpp);
-    if (prm.grid_w > 0) {
-        int tyi, txi;
-        if (prm.band_rows > 1) {        // bands of band_rows tile rows, column by column inside a band: vertically adjacent tiles follow each other
-            const int bsz = prm.tiles_x * prm.band_rows, band = r / bsz, rem = r - band * bsz;
-            const int rows = min(prm.band_rows, prm.tiles_y - band * prm.band_rows);
-            txi = rem / rows; tyi = band * prm.band_rows + (rem - txi * rows);
-        } else { tyi = r / prm.tiles_x; txi = r - tyi * prm.tiles_x; }
-        tc.ty0 = tyi * 8; tc.tx0 = txi * 8; tc.n0 = 0; tc.cnt = TILE;
-    }
-    else { tc.n0 = r * TILE; tc.cnt = min(TILE, prm.N - tc.n0); tc.tx0 = tc.ty0 = 0; }
-    return tc;
-}
-
 template <int NCH, bool FLY, int MODE, int KBLK = 4>
 __global__ void __launch_bounds__(THREADS, 1)
 lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams prm)
@@ -103,23 +53,12 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
     constexpr int NST = SM::NST, NREC = SM::NREC;
     // KBLK = K / 32 basis blocks actually present (K = 128, 64 or 32).  The smem / TMEM geometry stays that of K = 128 (M = 128 rows of D,
     // 32-KB stages); blocks >= KBLK are never loaded, read by the SIMT loops or drained, and the [v | t] block of R follows the last one.
-    constexpr int KR = 32 * KBLK, EXTB = KBLK, NMMA = KBLK == 4 ? NN : KR + 16;
+    constexpr int KR = 32 * KBLK, NMMA = KBLK == 4 ? NN : KR + 16;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // align through the 32-bit shared address so that the compiler keeps every access in the shared state space (LDS/STS, not generic LD/ST)
     unsigned char* base = smem_raw + (SM::slack ? ((512u - (smem_u32(smem_raw) & 511u)) & 511u) : 0u);
     if (SM::slack == 0 && (smem_u32(smem_raw) & 511u)) __trap();      // fail loudly: swizzle atoms need 512-B aligned stage bases
-    uint64_t* bars = reinterpret_cast<uint64_t*>(base + SM::off_bar);
-    uint64_t* fullB = bars;            // [NST]  TMA landed
-    uint64_t* rfree = bars + 4;        //        MMAs of the tile completed
-    uint64_t* flushb = bars + 5;       //        every MMA of the span completed
-    uint64_t* tmemfree = bars + 6;     //        lo accumulator drained
-    uint64_t* chain_done = bars + 7;   // [2]
-    uint64_t* drained = bars + 9;      // [2]
-    uint64_t* recs = bars + 11;        // [NREC] records of the tile in buffer s written (count W0)
-    uint64_t* gath = bars + 14;        // [NREC] M,q of the tile in buffer s written (count GW)
-    uint64_t* recfree = bars + 17;     // [NREC] records of the tile in buffer s consumed by the algebra warps (count AW)
-    uint64_t* rbdump = bars + 20;      //        gather warps parked their rbar partials (count GW)
-    uint64_t* rbfree = bars + 21;      //        algebra warps consumed them (count AW)
+    const Barriers bar(reinterpret_cast<uint64_t*>(base + SM::off_bar));
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(base + SM::off_tmem);
     int* sTile = reinterpret_cast<int*>(base + SM::off_tile);
     float* sPose = reinterpret_cast<float*>(base + SM::off_pose);
@@ -137,25 +76,10 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
     const int ntiles = (int)(t_end - t_begin);
 
     if (tid == 0) {
-        for (int i = 0; i < NST; ++i) mbar_init(&fullB[i], 1);
-        for (int i = 0; i < NREC; ++i) { mbar_init(&recs[i], W0); mbar_init(&gath[i], GW); mbar_init(&recfree[i], AW); }
-        mbar_init(rfree, 1); mbar_init(flushb, 1); mbar_init(tmemfree, DW);
-        mbar_init(&chain_done[0], 1); mbar_init(&chain_done[1], 1); mbar_init(&drained[0], DW); mbar_init(&drained[1], DW);
-        mbar_init(rbdump, GW); mbar_init(rbfree, AW);
-        fence_barrier_init();
+        init_barriers<NST, NREC>(bar);
         prefetch_tmap(&tmapB);
     }
-    if (warp == 0) tmem_alloc<TMEM_COLS>(s_tmem);
-    for (int i = tid; i < TILE * 8; i += THREADS) {       // pad chunks of R / R_lo's 5th block stay zero
-        const int r = i >> 3, c = i & 7;
-        *reinterpret_cast<float4*>(base + SM::off_R + EXTB * 8192 + sw128_32b_off(r, c)) = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (MODE == 3) *reinterpret_cast<float4*>(base + SM::off_Rlo + EXTB * 8192 + sw128_32b_off(r, c)) = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    fence_proxy_async_smem();
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem = *s_tmem;
+    const uint32_t tmem = setup_tmem<MODE, KBLK>(base + SM::off_R, base + SM::off_Rlo, s_tmem, tid, warp);
 
     // lane -> (row r of the warp's 16, half hf of the 128 basis columns); 16-B chunk walk rotated by the row so that every
     // quarter-warp touches 8 distinct bank groups of the swizzled tile (used by the b.W and the R-row loops)
@@ -178,33 +102,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
             else if (grid2d) { nxt.tx0 += 8; if (nxt.tx0 >= prm.tiles_x * 8) { nxt.tx0 = 0; nxt.ty0 += 8; } }
             else { nxt.n0 += TILE; nxt.cnt = min(TILE, N - nxt.n0); }
             const int b = tc.b;
-            if (gwi == 1 && j + 2 < ntiles) {             // L2 prefetch of the streaming inputs (conv1, p, D) two tiles ahead
-                const TileCoord tn = tile_coord(prm, t_begin + j + 2);
-                if (grid2d) {
-                    if (lane < 8) {
-                        const int gy = tn.ty0 + lane;
-                        if (gy < prm.grid_h && tn.tx0 < prm.grid_w) {
-                            const size_t n = (size_t)gy * prm.grid_w + tn.tx0;
-                            const int wpx = min(8, prm.grid_w - tn.tx0);
-                            prefetch_l2_bulk(prm.conv1 + ((size_t)tn.b * N + n) * C, (uint32_t)(wpx * C * 4));
-                            if ((n & 3) == 0 && (N & 3) == 0) {
-                                const uint32_t by = (uint32_t)(((wpx * 4) + 15) & ~15);
-                                prefetch_l2_bulk(prm.D + (size_t)tn.b * N + n, by);
-#pragma unroll
-                                for (int k = 0; k < 3; ++k) prefetch_l2_bulk(prm.p + ((size_t)tn.b * 3 + k) * N + n, by);
-                            }
-                        }
-                    }
-                } else if (lane == 0) {
-                    prefetch_l2_bulk(prm.conv1 + ((size_t)tn.b * N + tn.n0) * C, (uint32_t)(tn.cnt * C * 4));
-                    if ((N & 3) == 0) {
-                        const uint32_t by = (uint32_t)(((tn.cnt * 4) + 15) & ~15);
-                        prefetch_l2_bulk(prm.D + (size_t)tn.b * N + tn.n0, by);
-#pragma unroll
-                        for (int k = 0; k < 3; ++k) prefetch_l2_bulk(prm.p + ((size_t)tn.b * 3 + k) * N + tn.n0, by);
-                    }
-                }
-            }
+            if (gwi == 1 && j + 2 < ntiles) prefetch_inputs<C>(prm, tile_coord(prm, t_begin + j + 2), grid2d, N, lane);
             if (b != geom_b) {
                 geom_b = b;
                 __syncwarp();
@@ -213,7 +111,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                 else if (lane < 16) myPose[lane] = prm.intr[b * 4 + lane - 12];
                 if (KBLK == 4 || 4 * lane < KR)
                     *reinterpret_cast<float4*>(myW + 4 * lane) = __ldg(reinterpret_cast<const float4*>(prm.W + (size_t)b * KR + 4 * lane));
-                if constexpr (MODE == 1)     // a pure function of the inputs that changes whenever the iterate changes (see the rounding below)
+                if constexpr (MODE == 1)     // a pure function of the inputs that changes whenever the iterate changes (see tf32_stochastic4)
                     dseed = (__float_as_uint(__ldg(prm.W + (size_t)b * KR)) * 0x9E3779B1u) ^ (__float_as_uint(__ldg(prm.W + (size_t)b * KR + 1)) * 0x85EBCA77u)
                           ^ (__float_as_uint(__ldg(prm.W + (size_t)b * KR + 2)) * 0xC2B2AE3Du) ^ __float_as_uint(__ldg(prm.T + b * 3)) ^ (uint32_t)b;
                 __syncwarp();
@@ -230,10 +128,8 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                 p0 = __ldg(pp); p1 = __ldg(pp + N); p2 = __ldg(pp + 2 * (size_t)N);
                 D0 = __ldg(prm.D + (size_t)b * N + n);
             }
-            if (gwi == 0) TC6_TRACE(2, j, 0);
-            mbar_wait_parked(&recfree[sr], ((j / NREC) & 1) ^ 1);
-            mbar_wait_parked(&fullB[s], (j / NST) & 1);
-            if (gwi == 0) TC6_TRACE(2, j, 1);
+            mbar_wait_parked(&bar.recfree[sr], ((j / NREC) & 1) ^ 1);
+            mbar_wait_parked(&bar.fullB[s], (j / NST) & 1);
             float mydot;
             {
                 float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -244,45 +140,16 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                     const float4 bv = *reinterpret_cast<const float4*>(As + blk * 8192 + sw128_32b_off(nlr, c));
                     const float4 w4 = *reinterpret_cast<const float4*>(myW + blk * 32 + c * 4);
                     acc.x = fmaf(bv.x, w4.x, acc.x); acc.y = fmaf(bv.y, w4.y, acc.y); acc.z = fmaf(bv.z, w4.z, acc.z); acc.w = fmaf(bv.w, w4.w, acc.w);
-                    if constexpr (MODE == 1) {
-                        // single-pass mode: round the basis tile to tf32 IN PLACE.  The tensor core would truncate it (biased: relH 1e-5);
-                        // round-to-nearest is unbiased per launch (relH < 1e-6) but is the SAME perturbation of the basis at every LM
-                        // iteration, so its effect adds up coherently over a solve (W off by 1e-3 after 20 iterations).  Stochastic rounding
-                        // with a dither hashed from (iterate, pixel, column) is unbiased AND changes with the iterate, like the rounding
-                        // of R does; it is a pure function of the inputs, so results stay bit-reproducible.
-                        uint32_t hsh = dseed ^ ((uint32_t)n * 0x9E3779B1u) ^ ((uint32_t)(blk * 8 + c) * 0x85EBCA77u);
-                        hsh ^= hsh >> 16; hsh *= 0x7FEB352Du; hsh ^= hsh >> 15;
-                        uint32_t hs2 = hsh * 0x846CA68Bu; hs2 ^= hs2 >> 16;
+                    if constexpr (MODE == 1)     // single-pass mode: round the basis tile to tf32 IN PLACE (the tensor core would truncate it)
                         *reinterpret_cast<float4*>(const_cast<unsigned char*>(As) + blk * 8192 + sw128_32b_off(nlr, c)) =
-                            make_float4(__uint_as_float((__float_as_uint(bv.x) + (hsh & 0x1fffu)) & 0xFFFFE000u),
-                                        __uint_as_float((__float_as_uint(bv.y) + ((hsh >> 13) & 0x1fffu)) & 0xFFFFE000u),
-                                        __uint_as_float((__float_as_uint(bv.z) + (hs2 & 0x1fffu)) & 0xFFFFE000u),
-                                        __uint_as_float((__float_as_uint(bv.w) + ((hs2 >> 13) & 0x1fffu)) & 0xFFFFE000u));
-                    }
+                            tf32_stochastic4(bv, dseed ^ ((uint32_t)n * 0x9E3779B1u) ^ ((uint32_t)(blk * 8 + c) * 0x85EBCA77u));
                 }
                 if constexpr (MODE == 1) fence_proxy_async_smem();      // the MMA reads this stage through the async proxy
                 mydot = (acc.x + acc.y) + (acc.z + acc.w);
                 mydot += __shfl_xor_sync(0xffffffffu, mydot, 16);
             }
-            if (gwi == 0) TC6_TRACE(2, j, 2);
-            if (lane < 16) {                                 // thread per pixel (bundlenet.py:208-224, mask :231)
-                const float* pose = myPose;
-                float mask = 0.f, x = 0.f, y = 0.f, iZ = 0.f, rx = 0.f, ry = 0.f, rz = 0.f, dx = 0.f, dy = 0.f;
-                int x0 = 0, y0 = 0;
-                if (valid) {
-                    const float Dt = D0 + mydot;
-                    rx = pose[0] * p0 + pose[1] * p1 + pose[2] * p2;
-                    ry = pose[3] * p0 + pose[4] * p1 + pose[5] * p2;
-                    rz = pose[6] * p0 + pose[7] * p1 + pose[8] * p2;
-                    const float X = rx * Dt + pose[9], Y = ry * Dt + pose[10], Z = rz * Dt + pose[11];
-                    x = X / Z; y = Y / Z; iZ = 1.0f / Z;
-                    const float u = pose[12] * x + pose[14], v = pose[13] * y + pose[15];
-                    if ((u >= 0.f) && (u <= (float)(w - 1)) && (v >= 0.f) && (v <= (float)(h - 1)) && isfinite(iZ)) {
-                        mask = 1.f;
-                        const float fu = floorf(u), fv = floorf(v);
-                        x0 = (int)fu; y0 = (int)fv; dx = u - fu; dy = v - fv;
-                    }
-                }
+            if (lane < 16) {                                 // thread per pixel
+                const auto [mask, x, y, iZ, rx, ry, rz, dx, dy, x0, y0] = project_pixel(myPose, p0, p1, p2, D0, mydot, valid, w, h);
                 uint32_t o[4], cx[2] = {0u, 0u};
                 if constexpr (FLY) {                             // rows y0-1 .. y0+2 as float offsets, columns x0-1 .. x0+2 as packed pixel indices
                     o[0] = (uint32_t)(reflect_i(y0 - 1, h) * w * c2); o[1] = (uint32_t)(y0 * w * c2);
@@ -330,8 +197,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
             }
             if (gwi == 0 && lane == 0) sTile[sr * 4] = b;
             __syncwarp();
-            if (gwi == 0) TC6_TRACE(2, j, 3);
-            if (lane == 0) mbar_arrive(&recs[sr]);
+            if (lane == 0) mbar_arrive(&bar.recs[sr]);
         }
     } else if (warp < W0 + GW) {
         // ===================================================================== gather warps: records -> taps -> M, q
@@ -350,7 +216,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
         const uint64_t pol_tap = prm.l2_hints >= 2 ? l2_policy_evict_last() : l2_policy_evict_normal();
 
         auto dump_rb = [&]() {
-            if (ndump > 0) mbar_wait_parked(rbfree, (ndump - 1) & 1);       // the algebra warps consumed the previous hand-over
+            if (ndump > 0) mbar_wait_parked(bar.rbfree, (ndump - 1) & 1);       // the algebra warps consumed the previous hand-over
 #pragma unroll
             for (int u = 0; u < NCH * 4; ++u) rb[u] += __shfl_xor_sync(0xffffffffu, rb[u], 16);
             if (hw == 0) {
@@ -359,7 +225,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                     *reinterpret_cast<float4*>(sRbs + g * 128 + 64 * j + 4 * hl) = make_float4(rb[4 * j], rb[4 * j + 1], rb[4 * j + 2], rb[4 * j + 3]);
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive(rbdump);
+            if (lane == 0) mbar_arrive(bar.rbdump);
 #pragma unroll
             for (int u = 0; u < NCH * 4; ++u) rb[u] = 0.f;
             ++ndump;
@@ -367,9 +233,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
 
         for (int j = 0; j < ntiles; ++j) {
             const int s = j % NREC;
-            if (g == 0) TC6_TRACE(0, j, 0);
-            mbar_wait_parked(&recs[s], (j / NREC) & 1);
-            if (g == 0) TC6_TRACE(0, j, 1);
+            mbar_wait_parked(&bar.recs[s], (j / NREC) & 1);
             const int b = sTile[s * 4];
             if (b != cur_b) { if (cur_b >= 0) dump_rb(); cur_b = b; }
             float* rec = sRec + (s * TILE + g * PXW) * REC;
@@ -445,8 +309,7 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                 }
             }
             __syncwarp();
-            if (g == 0) TC6_TRACE(0, j, 2);
-            if (lane == 0) mbar_arrive(&gath[s]);
+            if (lane == 0) mbar_arrive(&bar.gath[s]);
         }
         if (cur_b >= 0) dump_rb();
     } else if (warp < W0 + GW + AW) {
@@ -455,7 +318,6 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
         const int awi = warp - (W0 + GW);                    // 0..3: pixels / rows 16*awi .. 16*awi+15
         const int atid = tid - (W0 + GW) * 32;
         const int nlr = awi * 16 + r16;
-        const SlotLayout L{KR, C};
         unsigned char* Rs = base + SM::off_R;
         float cc[28];
 #pragma unroll
@@ -473,41 +335,17 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
         auto issue_tma = [&](int t) {                        // basis tile t -> stage t % NST (elected thread)
             const int st = t % NST;
             const TileCoord tc = tile_coord(prm, t_begin + t);
-            mbar_arrive_expect_tx(&fullB[st], KBLK * 8192);
+            mbar_arrive_expect_tx(&bar.fullB[st], KBLK * 8192);
             unsigned char* dst = base + SM::off_A + st * STAGE_A;
             if (grid2d) {
 #pragma unroll
-                for (int blk = 0; blk < KBLK; ++blk) tma_load_3d_hint(dst + blk * 8192, &tmapB, blk * 32, tc.tx0, tc.b * prm.grid_h + tc.ty0, &fullB[st], pol_basis);
+                for (int blk = 0; blk < KBLK; ++blk) tma_load_3d_hint(dst + blk * 8192, &tmapB, blk * 32, tc.tx0, tc.b * prm.grid_h + tc.ty0, &bar.fullB[st], pol_basis);
             } else {
                 const int row = tc.b * N + tc.n0;
 #pragma unroll
-                for (int blk = 0; blk < KBLK; ++blk) tma_load_2d_hint(dst + blk * 8192, &tmapB, blk * 32, row, &fullB[st], pol_basis);
+                for (int blk = 0; blk < KBLK; ++blk) tma_load_2d_hint(dst + blk * 8192, &tmapB, blk * 32, row, &bar.fullB[st], pol_basis);
             }
         };
-        auto flush = [&](int sp) {
-            float* slot = prm.partials + ((size_t)blockIdx.x * prm.max_span + sp) * prm.slot_floats;
-            // H_cc / g_c / nvalid: 16 pixel-lanes -> warp total (fixed shuffle tree) -> 4 warp partials summed in fixed order
-#pragma unroll
-            for (int q = 0; q < 28; ++q) {
-                float v = cc[q];
-                v += __shfl_xor_sync(0xffffffffu, v, 8); v += __shfl_xor_sync(0xffffffffu, v, 4);
-                v += __shfl_xor_sync(0xffffffffu, v, 2); v += __shfl_xor_sync(0xffffffffu, v, 1);
-                if (lane == 0) sCcs[awi * 28 + q] = v;
-                cc[q] = 0.f;
-            }
-            mbar_wait_parked(rbdump, sp & 1);                // the gather warps parked their |diff| sums for this pair
-            team_bar<AW * 32>();
-            if (atid < C) {
-                float sum = 0.f;
-#pragma unroll
-                for (int wq = 0; wq < GW; ++wq) sum += sRbs[wq * 128 + atid];
-                slot[L.off_rbar() + atid] = sum;
-            }
-            if (atid < 28) slot[L.off_cc() + atid] = (sCcs[atid] + sCcs[28 + atid]) + (sCcs[56 + atid] + sCcs[84 + atid]);
-            team_bar<AW * 32>();
-            if (lane == 0) mbar_arrive(rbfree);
-        };
-
         if (awi == 0 && lane == 0)
             for (int t = 0; t < NST && t < ntiles; ++t) issue_tma(t);      // every stage starts free
 
@@ -516,60 +354,20 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
             const bool last_of_pair = (++rr == prm.tiles_per_pair) || (j == ntiles - 1);
             if (rr == prm.tiles_per_pair) rr = 0;
             const unsigned char* As = base + SM::off_A + s * STAGE_A;
-            if (awi == 0) TC6_TRACE(1, j, 0);
-            mbar_wait_parked(&gath[sr], (j / NREC) & 1);
-            if (awi == 0) TC6_TRACE(1, j, 1);
+            mbar_wait_parked(&bar.gath[sr], (j / NREC) & 1);
             const int b = sTile[sr * 4];
             if (b != scale_b) { scale_b = b; ++sspan; fx = __ldg(prm.intr + b * 4); fy = __ldg(prm.intr + b * 4 + 1); }
             float ext[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-            if (lane < 16) {                                 // thread per pixel (bundlenet.py:49-74)
-                const float* rec = sRec + (sr * TILE + nlr) * REC;
-                const float4 ra = *reinterpret_cast<const float4*>(rec + 12), rbq = *reinterpret_cast<const float4*>(rec + 4),
-                             rc = *reinterpret_cast<const float4*>(rec + 8);
-                if (rbq.x != 0.f) {
-                    const float m11 = ra.x, m12 = ra.y, m22 = ra.z, q1 = ra.w, q2 = rc.w, x = rbq.y, y = rbq.z, iZ = rbq.w;
-                    const float rx = rc.x, ry = rc.y, rz = rc.z;
-                    const float a0[6] = {-fx * (x * y), -fx * (-1.f - x * x), -fx * y, -fx * (-iZ), 0.f, -fx * (x * iZ)};
-                    const float a1[6] = {-fy * (1.f + y * y), -fy * (-(x * y)), -fy * (-x), 0.f, -fy * (-iZ), -fy * (y * iZ)};
-                    float ux[6], uy[6];
-#pragma unroll
-                    for (int i = 0; i < 6; ++i) { ux[i] = m11 * a0[i] + m12 * a1[i]; uy[i] = m12 * a0[i] + m22 * a1[i]; }
-                    int q = 0;
-#pragma unroll
-                    for (int i = 0; i < 6; ++i)
-#pragma unroll
-                        for (int jj = i; jj < 6; ++jj) { cc[q] += a0[i] * ux[jj] + a1[i] * uy[jj]; ++q; }
-#pragma unroll
-                    for (int i = 0; i < 6; ++i) cc[21 + i] += a0[i] * q1 + a1[i] * q2;
-                    cc[27] += 1.f;
-                    const float jd0 = fx * ((rx - rz * x) * iZ), jd1 = fy * ((ry - rz * y) * iZ);
-                    const float u0 = m11 * jd0 + m12 * jd1, u1 = m12 * jd0 + m22 * jd1;
-#pragma unroll
-                    for (int i = 0; i < 6; ++i) ext[i] = a0[i] * u0 + a1[i] * u1;
-                    ext[6] = jd0 * q1 + jd1 * q2;
-                    ext[7] = jd0 * u0 + jd1 * u1;
-                }
-            }
+            if (lane < 16) pixel_algebra(sRec + (sr * TILE + nlr) * REC, fx, fy, cc, ext);
             __syncwarp();
-            if (lane == 0) mbar_arrive(&recfree[sr]);        // the record buffer may be refilled (everything needed is in registers)
+            if (lane == 0) mbar_arrive(&bar.recfree[sr]);        // the record buffer may be refilled (everything needed is in registers)
             const float sn = __shfl_sync(0xffffffffu, ext[7], r16);   // s_n of this lane's row
-            if (awi == 0) TC6_TRACE(1, j, 2);
-            mbar_wait_parked(&fullB[s], (j / NST) & 1);      // long complete; orders the TMA writes before the reads below
+            mbar_wait_parked(&bar.fullB[s], (j / NST) & 1);  // long complete; orders the TMA writes before the reads below
             if (j > 0) {
-                mbar_wait_parked(rfree, (j - 1) & 1);        // MMAs of tile j-1 done: R / A_lo / R_lo and stage (j-1) % NST are free
+                mbar_wait_parked(bar.rfree, (j - 1) & 1);    // MMAs of tile j-1 done: R / A_lo / R_lo and stage (j-1) % NST are free
                 if (awi == 0 && lane == 0 && j - 1 + NST < ntiles) issue_tma(j - 1 + NST);
             }
-            if (awi == 0) TC6_TRACE(1, j, 3);
-            if (lane < 16) {                                 // R columns 128..134 = [v(6) | t], column 135 stays zero
-                const float4 e0 = make_float4(tf32_rna(ext[0]), tf32_rna(ext[1]), tf32_rna(ext[2]), tf32_rna(ext[3]));
-                const float4 e1 = make_float4(tf32_rna(ext[4]), tf32_rna(ext[5]), tf32_rna(ext[6]), 0.f);
-                *reinterpret_cast<float4*>(Rs + EXTB * 8192 + sw128_32b_off(nlr, 0)) = e0;
-                *reinterpret_cast<float4*>(Rs + EXTB * 8192 + sw128_32b_off(nlr, 1)) = e1;
-                if constexpr (MODE == 3) {
-                    *reinterpret_cast<float4*>(base + SM::off_Rlo + EXTB * 8192 + sw128_32b_off(nlr, 0)) = make_float4(ext[0] - e0.x, ext[1] - e0.y, ext[2] - e0.z, ext[3] - e0.w);
-                    *reinterpret_cast<float4*>(base + SM::off_Rlo + EXTB * 8192 + sw128_32b_off(nlr, 1)) = make_float4(ext[4] - e1.x, ext[5] - e1.y, ext[6] - e1.z, 0.f);
-                }
-            }
+            if (lane < 16) write_vt<MODE, KBLK>(Rs, base + SM::off_Rlo, nlr, ext);
             // R rows (and the split parts): elementwise on the lane's half row, so walk the PHYSICAL 16-B slots (rotated by the row: every
             // quarter-warp touches 8 distinct bank groups) and skip the swizzle arithmetic
             const uint32_t rowoff = hf * 16384 + nlr * 128;
@@ -589,12 +387,11 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                     *reinterpret_cast<float4*>(base + SM::off_Rlo + off) = make_float4(pv.x - hv.x, pv.y - hv.y, pv.z - hv.z, pv.w - hv.w);
             }
             fence_proxy_async_smem();
-            if (awi == 0) TC6_TRACE(1, j, 4);
             team_bar<AW * 32>();                           // all 64 rows written
             if (awi == 0) {
                 if (lane == 0) {                             // ---- tcgen05.mma issue for this tile
-                    if (new_span) { mbar_wait_parked(tmemfree, (mspan & 1) ^ 1); accL = 0; new_span = false; }
-                    if (tic == 0) { ++chain; set = chain & 1; mbar_wait_parked(&drained[set], ((chain >> 1) & 1) ^ 1); accH = 0; }
+                    if (new_span) { mbar_wait_parked(bar.tmemfree, (mspan & 1) ^ 1); accL = 0; new_span = false; }
+                    if (tic == 0) { ++chain; set = chain & 1; mbar_wait_parked(&bar.drained[set], ((chain >> 1) & 1) ^ 1); accH = 0; }
                     tc_fence_after_sync();
                     const uint32_t ahi = smem_u32(base + SM::off_A + s * STAGE_A);
                     const uint32_t rhi = smem_u32(base + SM::off_R), rlo = smem_u32(base + SM::off_Rlo), alo = smem_u32(base + SM::off_Alo);
@@ -610,95 +407,18 @@ lm_build_tc6_kernel(const __grid_constant__ CUtensorMap tmapB, const BuildParams
                             if (pass == 0) accH = 1; else accL = 1;
                         }
                     }
-                    mma_commit(rfree);
-                    if (++tic == CHAIN) { mma_commit(&chain_done[set]); tic = 0; }
-                    if (last_of_pair) { if (tic > 0) mma_commit(&chain_done[set]); mma_commit(flushb); ++mspan; tic = 0; new_span = true; }
+                    mma_commit(bar.rfree);
+                    if (++tic == CHAIN) { mma_commit(&bar.chain_done[set]); tic = 0; }
+                    if (last_of_pair) { if (tic > 0) mma_commit(&bar.chain_done[set]); mma_commit(bar.flushb); ++mspan; tic = 0; new_span = true; }
                 }
                 __syncwarp();
             }
-            if (awi == 0) TC6_TRACE(1, j, 5);
-            if (last_of_pair) flush(sspan);
+            if (last_of_pair) flush<KBLK, C>(prm, bar, cc, sspan, sCcs, sRbs, awi, atid, lane);
         }
     } else {
-        // ===================================================================== drainer warps: TMEM -> partial slots, fully asynchronous
-        setmaxnreg_dec<32>();
-        const int dq = warp - (W0 + GW + AW);                // TMEM lane quadrant (= warp % 4)
-        const SlotLayout L{KR, C};
-        // The CTA's partial slot (<= 2 x 68 KB) is read-modify-written once per chain of CHAIN tiles.  Left to the default policy the streaming
-        // inputs push it out of L2 between two chains: ncu showed 1.3 GB of DRAM writes per launch (and as many reads) for a kernel that writes
-        // 20 MB of results.  evict-last keeps the 20 MB of slots of all CTAs resident.
-        const uint64_t pol_slot = l2_policy_evict_last();
-        auto drain_region = [&](float* slot, uint32_t col0, bool overwrite) {
-            const int row = dq * 32 + lane;
-            if (KBLK != 4 && dq * 32 >= KR) return;          // this lane quadrant holds no basis row (warp-uniform)
-            const uint32_t tq = tmem + ((uint32_t)(dq * 32) << 16) + col0;
-            float v[16];
-#pragma unroll 1
-            for (int cb = 0; cb < KR / 16; ++cb) {
-                tmem_ld_32x16(tq + cb * 16, v);
-                float* dst = slot + (size_t)(cb * 16) * KR + row;
-                if (overwrite) {
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) st_f32_hint(dst + (size_t)j * KR, v[j], pol_slot);
-                } else {
-#pragma unroll
-                    for (int hb = 0; hb < 16; hb += 8) {     // 8 columns at a time: the drainers live on 32 registers
-                        float o[8];
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) o[j] = ld_f32_hint(dst + (size_t)(hb + j) * KR, pol_slot);
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) st_f32_hint(dst + (size_t)(hb + j) * KR, o[j] + v[hb + j], pol_slot);
-                    }
-                }
-            }
-            tmem_ld_32x16(tq + KR, v);
-            float* dst = slot + L.off_ext() + row;
-#pragma unroll
-            for (int r = 0; r < 7; ++r) {
-                if (overwrite) st_f32_hint(dst + r * KR, v[r], pol_slot);
-                else st_f32_hint(dst + r * KR, ld_f32_hint(dst + r * KR, pol_slot) + v[r], pol_slot);
-            }
-        };
-        int chain = -1, tic = 0, span = 0, cur_b = -1;
-        bool first = true;
-        int b = (ntiles > 0) ? (int)((unsigned)t_begin / (unsigned)prm.tiles_per_pair) : 0;
-        int rr = (ntiles > 0) ? (int)((unsigned)t_begin - (unsigned)b * (unsigned)prm.tiles_per_pair) : 0;
-        auto drain_hi = [&]() {
-            const int set = chain & 1;
-            float* slot = prm.partials + ((size_t)blockIdx.x * prm.max_span + span) * prm.slot_floats;
-            mbar_wait_parked(&chain_done[set], (chain >> 1) & 1);
-            tc_fence_after_sync();
-            drain_region(slot, set * NN, first);
-            first = false;
-            tc_fence_before_sync();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&drained[set]);
-        };
-        auto end_span = [&]() {
-            if (tic > 0) drain_hi();
-            if constexpr (MODE >= 2) {
-                float* slot = prm.partials + ((size_t)blockIdx.x * prm.max_span + span) * prm.slot_floats;
-                mbar_wait_parked(flushb, span & 1);
-                tc_fence_after_sync();
-                drain_region(slot, ACCL, false);
-                tc_fence_before_sync();
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(tmemfree);
-            ++span;
-        };
-        for (int it = 0; it < ntiles; ++it) {
-            if (b != cur_b) { if (cur_b >= 0) end_span(); cur_b = b; tic = 0; first = true; }
-            if (tic == 0) ++chain;
-            if (++tic == CHAIN) { drain_hi(); tic = 0; }
-            if (++rr == prm.tiles_per_pair) { rr = 0; ++b; }
-        }
-        if (cur_b >= 0) end_span();
+        drainer_role<32, MODE, KBLK, C>(prm, bar, tmem, t_begin, ntiles, warp - (W0 + GW + AW), lane);
     }
-
-    tc_fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TMEM_COLS>(tmem);
+    release_tmem(tmem, warp);
 }
 
 template <int NCH, bool FLY, int MODE, int KBLK = 4>

@@ -1,8 +1,8 @@
 // lm_build_tc7.cu — tensor-core build kernel, generation 7: the F2 footprint of every 8x8 tile is staged into shared memory by TMA.
 //
 // Applies to the F2-only conv2 layout on a dense pixel grid (the BundleResize boundary: feature maps in, gradients derived on the fly,
-// reference bundlenet.py:92-100, 385-389).  Same contract, slot layout, tensor-core contraction and precision modes as generation 6
-// (lm_build_tc6.cu; lm_build_tc_host.cu has the overview); what changes is where the 12 taps per pixel and channel come from:
+// reference bundlenet.py:92-100, 385-389).  Same contract, slot layout, tensor-core contraction, precision modes and pipeline roles as generation 6
+// (lm_build_tc_roles.cuh; lm_build_tc_host.cu has the overview); what changes is where the 12 taps per pixel and channel come from:
 //
 //   generation 6: 13 x ld.global.nc per (pixel, 4 channels), latency-bound (ncu r01b: long-scoreboard 65% of the issue interval, 0.75
 //                 eligible warps per scheduler) and every texel fetched ~1.3x (L1) with 12 x the LSU traffic on the L1/L2 path;
@@ -22,61 +22,35 @@
 //                 algebra warps did in generation 6; the geometry warps only form b.W and the warp; the per-channel arithmetic runs on packed
 //                 fp32 pairs (FFMA2 / FMUL2 / FADD2); conv1 arrives with the window (one 4-D TMA box {32 ch, 8, 8, pair} per chunk).
 //
-// Roles (896 threads, 1 CTA / SM) and barriers as generation 6, plus winfull[NWB] (TMA landed, count 1 + tx) / winfree[NWB] (count GW).
-#include "common.cuh"
-#include "lm_build.h"
-#include "tc_utils.cuh"
+// Register budgets 48 / 88 / 64 / 40 (geometry / gather / algebra / drainers); the window ring adds winfull[NWB] (TMA landed, count 1 + tx) /
+// winfree[NWB] (count GW) to the barriers.
+#include "lm_build_tc_roles.cuh"
 #include "tmap.h"
 #include <limits.h>
 
 namespace banet { namespace v7 {
-using namespace tc;
+using namespace tcb;
 
-constexpr int TILE = 64, W0 = 4, GW = 16, AW = 4, DW = 4;      // geometry | gather | algebra | drainer warps
-constexpr int THREADS = (W0 + GW + AW + DW) * 32;               // 896
-constexpr int NN = 160;
-constexpr int STAGE_A = 4 * TILE * 128, STAGE_R = 5 * TILE * 128;
-constexpr int REC = 16;
-constexpr int CHAIN = 8, TMEM_COLS = 512, ACCL = 320;
-#ifndef BANET_TC7_WX
-#define BANET_TC7_WX 13
-#endif
-#ifndef BANET_TC7_WY
-#define BANET_TC7_WY 13
-#endif
-#ifndef BANET_TC7_NWB
-#define BANET_TC7_NWB 2
-#endif
-#ifndef BANET_TC7_NST1
-#define BANET_TC7_NST1 3
-#endif
 constexpr int CHK = 32;                                         // channels per staged chunk: one texel chunk = 128 B = all 32 banks
-constexpr int WX = BANET_TC7_WX, WY = BANET_TC7_WY;             // staged window (texels); an 8x8 tile needs >= 11..12 at unit zoom
+constexpr int WX = 13, WY = 13;                                 // staged window (texels); an 8x8 tile needs >= 11..12 at unit zoom
 constexpr int WIN_BYTES = WX * WY * CHK * 4;
-#ifdef BANET_TC7_DBG_BOXY            // timing experiment only: the TMA box has fewer rows than the window (results are garbage)
-constexpr int BOX_Y = BANET_TC7_DBG_BOXY;
-#else
-constexpr int BOX_Y = WY;
-#endif
-constexpr int WIN_TX_BYTES = WX * BOX_Y * CHK * 4;
 constexpr int C1_BYTES = TILE * CHK * 4;                        // conv1 chunk of the tile: [8][8] pixels x 32 channels, pixel-major 128-B rows
 constexpr int WBUF = WIN_BYTES + C1_BYTES;                      // one ring buffer = F2 window chunk + conv1 chunk
 
 template <int MODE, int NCH> struct Smem {
     static_assert(MODE == 1 || MODE == 2, "generation 7 implements TF32X1 and TF32X2 (TF32X3 stays on generation 6: no room for the windows)");
-    static constexpr int NST = MODE == 1 ? BANET_TC7_NST1 : 2;
+    static constexpr int NST = MODE == 1 ? 3 : 2;
     static constexpr int NREC = 3;
-    // window ring; never deeper than one tile's chunks (C/32): the producer may look ahead into tile j+1 only (a wait on the records of
+    // window ring; never deeper than one tile's chunks (C/32 >= 2): the producer may look ahead into tile j+1 only (a wait on the records of
     // tile j+2 from inside tile j could close a cycle through the basis ring: rfree(j) <- gath[j] <- the producer itself)
-    static constexpr int NWB = BANET_TC7_NWB < 2 * NCH ? BANET_TC7_NWB : 2 * NCH;
+    static constexpr int NWB = 2;
     static constexpr int off_A = 0;
     static constexpr int off_R = NST * STAGE_A;
     static constexpr int off_Alo = off_R + STAGE_R;
-    static constexpr int off_Rlo = off_Alo + (MODE >= 2 ? STAGE_A : 0);      // (MODE 3 only; kept so that the shared algebra code compiles)
-    static constexpr int off_win = off_Rlo;                            // [NWB] x ([WY][WX][32] floats F2 window chunk | [64][32] floats conv1 chunk)
+    static constexpr int off_win = off_Alo + (MODE >= 2 ? STAGE_A : 0);      // [NWB] x ([WY][WX][32] floats F2 window chunk | [64][32] floats conv1 chunk)
     static constexpr int off_misc = off_win + NWB * WBUF;
-    static constexpr int off_bar = off_misc;                           // 22 + 2*NWB mbarriers (<= 30)
-    static constexpr int off_tmem = off_bar + 30 * 8;
+    static constexpr int off_bar = off_misc;                           // NBARS + 2*NWB mbarriers (<= 30)
+    static constexpr int off_tmem = off_bar + (NBARS + 8) * 8;
     static constexpr int off_tile = off_misc + 256;                    // [NREC][8] ints: pair, tx0, ty0, fx, fy (float bits), dither seed of the tile in record buffer s
     static constexpr int off_box = off_tile + 128;                     // [NREC][W0][4] ints: tap bounding box (xmin,xmax,ymin,ymax) per geometry warp
     static constexpr int off_pose = off_box + NREC * W0 * 16;          // [W0][16] floats (private to each geometry warp)
@@ -91,14 +65,6 @@ template <int MODE, int NCH> struct Smem {
     static_assert(bytes <= 232448, "shared memory budget of one sm_100 CTA");
 };
 
-template <int NT> __device__ __forceinline__ void team_bar() { asm volatile("bar.sync 2, %0;" :: "n"(NT) : "memory"); }
-__device__ __forceinline__ int reflect_i(int i, int n) { i = i < 0 ? -i : (i >= n ? 2 * n - 2 - i : i); return i < 0 ? 0 : i; }
-__device__ __forceinline__ float4 ldg4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
-__device__ __forceinline__ float4 lds4(uint32_t saddr) {
-    float4 r;
-    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(saddr));
-    return r;
-}
 // packed fp32 pairs (sm_100: FFMA2 / FMUL2 / FADD2, one issue slot for two lanes' worth of channels; a (w, w) pair is encoded as a scalar broadcast)
 typedef unsigned long long u64;
 __device__ __forceinline__ u64 pk2(float a, float b) { u64 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a), "f"(b)); return r; }
@@ -120,9 +86,8 @@ __device__ __forceinline__ float qsum8(float v) {               // sum over the 
     v += __shfl_xor_sync(0xffffffffu, v, 4); v += __shfl_xor_sync(0xffffffffu, v, 2); v += __shfl_xor_sync(0xffffffffu, v, 1);
     return v;
 }
-struct TileCoord { int b, n0, cnt, tx0, ty0; };
-// tile index -> (pair, 8x8 patch): bands of prm.band_rows tile rows, column by column inside a band
-__device__ __forceinline__ TileCoord tile_coord(const BuildParams& prm, long long tl) {
+// tile index -> (pair, 8x8 patch): bands of prm.band_rows tile rows, column by column inside a band (the dense-grid, banded case of tile_coord)
+__device__ __forceinline__ TileCoord banded_tile_coord(const BuildParams& prm, long long tl) {
     TileCoord tc;
     const unsigned t = (unsigned)tl, tpp = (unsigned)prm.tiles_per_pair;
     tc.b = (int)(t / tpp);
@@ -135,7 +100,7 @@ __device__ __forceinline__ TileCoord tile_coord(const BuildParams& prm, long lon
     return tc;
 }
 
-// incremental form of tile_coord (no integer divisions per tile): walks the same band order
+// incremental form of banded_tile_coord (no integer divisions per tile): walks the same band order
 struct TileStepper {
     int b, r, band, txi, tyr, rows;              // pair, tile index inside the pair, band, tile column, row inside the band, rows of the band
     __device__ __forceinline__ void init(const BuildParams& prm, long long tl) {
@@ -162,24 +127,14 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
 {
     using SM = Smem<MODE, NCH>;
     constexpr int NST = SM::NST, NREC = SM::NREC, NWB = SM::NWB;
-    constexpr int KR = 32 * KBLK, EXTB = KBLK, NMMA = KBLK == 4 ? NN : KR + 16;
+    constexpr int KR = 32 * KBLK, NMMA = KBLK == 4 ? NN : KR + 16;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // align through the 32-bit shared address so that the compiler keeps every access in the shared state space (LDS/STS, not generic LD/ST)
     unsigned char* base = smem_raw + ((512u - (smem_u32(smem_raw) & 511u)) & 511u);
     uint64_t* bars = reinterpret_cast<uint64_t*>(base + SM::off_bar);
-    uint64_t* fullB = bars;            // [NST]  TMA landed
-    uint64_t* rfree = bars + 4;        //        MMAs of the tile completed
-    uint64_t* flushb = bars + 5;       //        every MMA of the span completed
-    uint64_t* tmemfree = bars + 6;     //        lo accumulator drained
-    uint64_t* chain_done = bars + 7;   // [2]
-    uint64_t* drained = bars + 9;      // [2]
-    uint64_t* recs = bars + 11;        // [NREC] records of the tile in buffer s written (count W0)
-    uint64_t* gath = bars + 14;        // [NREC] M,q of the tile in buffer s written (count GW)
-    uint64_t* recfree = bars + 17;     // [NREC] records of the tile in buffer s consumed by the algebra warps (count AW)
-    uint64_t* rbdump = bars + 20;      //        gather warps parked their rbar partials (count GW)
-    uint64_t* rbfree = bars + 21;      //        algebra warps consumed them (count AW)
-    uint64_t* winfull = bars + 22;     // [NWB]  window chunk landed (count 1 + tx bytes; plain arrive for a direct-tap tile)
-    uint64_t* winfree = bars + 26;     // [NWB]  window chunk consumed by the gather warps (count GW)
+    const Barriers bar(bars);
+    uint64_t* winfull = bars + NBARS;        // [NWB]  window chunk landed (count 1 + tx bytes)
+    uint64_t* winfree = bars + NBARS + 4;    // [NWB]  window chunk consumed by the gather warps (count GW)
     uint32_t* s_tmem = reinterpret_cast<uint32_t*>(base + SM::off_tmem);
     int* sTile = reinterpret_cast<int*>(base + SM::off_tile);
     int* sBox = reinterpret_cast<int*>(base + SM::off_box);
@@ -191,32 +146,17 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int N = prm.N, h = prm.h, w = prm.w, c2 = prm.c2;
-    constexpr bool grid2d = true;
     constexpr int C = 64 * NCH;
     const long long t_begin = part_begin(prm.total_tiles, gridDim.x, blockIdx.x);
     const long long t_end   = part_begin(prm.total_tiles, gridDim.x, blockIdx.x + 1);
     const int ntiles = (int)(t_end - t_begin);
 
     if (tid == 0) {
-        for (int i = 0; i < NST; ++i) mbar_init(&fullB[i], 1);
-        for (int i = 0; i < NREC; ++i) { mbar_init(&recs[i], W0); mbar_init(&gath[i], GW); mbar_init(&recfree[i], AW); }
         for (int i = 0; i < NWB; ++i) { mbar_init(&winfull[i], 1); mbar_init(&winfree[i], GW); }
-        mbar_init(rfree, 1); mbar_init(flushb, 1); mbar_init(tmemfree, DW);
-        mbar_init(&chain_done[0], 1); mbar_init(&chain_done[1], 1); mbar_init(&drained[0], DW); mbar_init(&drained[1], DW);
-        mbar_init(rbdump, GW); mbar_init(rbfree, AW);
-        fence_barrier_init();
+        init_barriers<NST, NREC>(bar);
         prefetch_tmap(&tmapB); prefetch_tmap(&tmapF); prefetch_tmap(&tmapC);
     }
-    if (warp == 0) tmem_alloc<TMEM_COLS>(s_tmem);
-    for (int i = tid; i < TILE * 8; i += THREADS) {       // pad chunks of R's 5th block stay zero
-        const int r = i >> 3, c = i & 7;
-        *reinterpret_cast<float4*>(base + SM::off_R + EXTB * 8192 + sw128_32b_off(r, c)) = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    fence_proxy_async_smem();
-    tc_fence_before_sync();
-    __syncthreads();
-    tc_fence_after_sync();
-    const uint32_t tmem = *s_tmem;
+    const uint32_t tmem = setup_tmem<MODE, KBLK>(base + SM::off_R, nullptr, s_tmem, tid, warp);
 
     // lane -> (row r of the warp's 16, half hf of the 128 basis columns); 16-B chunk walk rotated by the row so that every
     // quarter-warp touches 8 distinct bank groups of the swizzled tile (used by the b.W and the R-row loops)
@@ -237,23 +177,7 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
             TileCoord tc; tc.b = cur.b; tc.tx0 = cur.tx0(); tc.ty0 = cur.ty0(prm); tc.n0 = 0; tc.cnt = TILE;
             cur.next(prm);
             const int b = tc.b;
-            if (gwi == 1 && j + 2 < ntiles) {             // L2 prefetch of the streaming inputs (conv1, p, D) two tiles ahead
-                const int atx = ahead.tx0(), aty = ahead.ty0(prm), ab = ahead.b;
-                if (lane < 8) {
-                    const int gy = aty + lane;
-                    if (gy < prm.grid_h && atx < prm.grid_w) {
-                        const size_t n = (size_t)gy * prm.grid_w + atx;
-                        const int wpx = min(8, prm.grid_w - atx);
-                        prefetch_l2_bulk(prm.conv1 + ((size_t)ab * N + n) * C, (uint32_t)(wpx * C * 4));
-                        if ((n & 3) == 0 && (N & 3) == 0) {
-                            const uint32_t by = (uint32_t)(((wpx * 4) + 15) & ~15);
-                            prefetch_l2_bulk(prm.D + (size_t)ab * N + n, by);
-#pragma unroll
-                            for (int k = 0; k < 3; ++k) prefetch_l2_bulk(prm.p + ((size_t)ab * 3 + k) * N + n, by);
-                        }
-                    }
-                }
-            }
+            if (gwi == 1 && j + 2 < ntiles) prefetch_inputs<C>(prm, TileCoord{ahead.b, 0, TILE, ahead.tx0(), ahead.ty0(prm)}, true, N, lane);
             ahead.next(prm);
             if (b != geom_b) {
                 geom_b = b;
@@ -263,7 +187,7 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                 else if (lane < 16) myPose[lane] = prm.intr[b * 4 + lane - 12];
                 if (KBLK == 4 || 4 * lane < KR)
                     *reinterpret_cast<float4*>(myW + 4 * lane) = __ldg(reinterpret_cast<const float4*>(prm.W + (size_t)b * KR + 4 * lane));
-                if constexpr (MODE == 1)     // a pure function of the inputs that changes whenever the iterate changes (see the rounding below)
+                if constexpr (MODE == 1)     // a pure function of the inputs that changes whenever the iterate changes (see tf32_stochastic4)
                     dseed = (__float_as_uint(__ldg(prm.W + (size_t)b * KR)) * 0x9E3779B1u) ^ (__float_as_uint(__ldg(prm.W + (size_t)b * KR + 1)) * 0x85EBCA77u)
                           ^ (__float_as_uint(__ldg(prm.W + (size_t)b * KR + 2)) * 0xC2B2AE3Du) ^ __float_as_uint(__ldg(prm.T + b * 3)) ^ (uint32_t)b;
                 __syncwarp();
@@ -280,8 +204,8 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                 p0 = __ldg(pp); p1 = __ldg(pp + N); p2 = __ldg(pp + 2 * (size_t)N);
                 D0 = __ldg(prm.D + (size_t)b * N + n);
             }
-            mbar_wait_parked(&recfree[sr], ((j / NREC) & 1) ^ 1);
-            mbar_wait_parked(&fullB[s], (j / NST) & 1);
+            mbar_wait_parked(&bar.recfree[sr], ((j / NREC) & 1) ^ 1);
+            mbar_wait_parked(&bar.fullB[s], (j / NST) & 1);
             float mydot;
             {
                 float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -297,24 +221,8 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                 mydot += __shfl_xor_sync(0xffffffffu, mydot, 16);
             }
             int bxmin = INT_MAX, bxmax = INT_MIN, bymin = INT_MAX, bymax = INT_MIN;
-            if (lane < 16) {                                 // thread per pixel (bundlenet.py:208-224, mask :231)
-                const float* pose = myPose;
-                float mask = 0.f, x = 0.f, y = 0.f, iZ = 0.f, rx = 0.f, ry = 0.f, rz = 0.f, dx = 0.f, dy = 0.f;
-                int x0 = 0, y0 = 0;
-                if (valid) {
-                    const float Dt = D0 + mydot;
-                    rx = pose[0] * p0 + pose[1] * p1 + pose[2] * p2;
-                    ry = pose[3] * p0 + pose[4] * p1 + pose[5] * p2;
-                    rz = pose[6] * p0 + pose[7] * p1 + pose[8] * p2;
-                    const float X = rx * Dt + pose[9], Y = ry * Dt + pose[10], Z = rz * Dt + pose[11];
-                    x = X / Z; y = Y / Z; iZ = 1.0f / Z;
-                    const float u = pose[12] * x + pose[14], v = pose[13] * y + pose[15];
-                    if ((u >= 0.f) && (u <= (float)(w - 1)) && (v >= 0.f) && (v <= (float)(h - 1)) && isfinite(iZ)) {
-                        mask = 1.f;
-                        const float fu = floorf(u), fv = floorf(v);
-                        x0 = (int)fu; y0 = (int)fv; dx = u - fu; dy = v - fv;
-                    }
-                }
+            if (lane < 16) {                                 // thread per pixel
+                const auto [mask, x, y, iZ, rx, ry, rz, dx, dy, x0, y0] = project_pixel(myPose, p0, p1, p2, D0, mydot, valid, w, h);
                 // rows y0-1 .. y0+2 and columns x0-1 .. x0+2 with the REFLECT-by-one border of grad_fixed (bundlenet.py:97), 16 bits each
                 const int ym = reflect_i(y0 - 1, h), y1 = reflect_i(y0 + 1, h), yp = reflect_i(y0 + 2, h);
                 const int xm = reflect_i(x0 - 1, w), x1 = reflect_i(x0 + 1, w), xp = reflect_i(x0 + 2, w);
@@ -337,7 +245,7 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                     sTile[sr * 8 + 3] = __float_as_int(myPose[12]); sTile[sr * 8 + 4] = __float_as_int(myPose[13]); sTile[sr * 8 + 5] = (int)dseed; }
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive(&recs[sr]);
+            if (lane == 0) mbar_arrive(&bar.recs[sr]);
         }
     } else if (warp < W0 + GW) {
         // ===================================================================== gather warps: records -> staged taps (LDS) -> M, q
@@ -352,7 +260,7 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
         const uint32_t win0 = smem_u32(base + SM::off_win);
 
         auto dump_rb = [&]() {
-            if (ndump > 0) mbar_wait_parked(rbfree, (ndump - 1) & 1);       // the algebra warps consumed the previous hand-over
+            if (ndump > 0) mbar_wait_parked(bar.rbfree, (ndump - 1) & 1);       // the algebra warps consumed the previous hand-over
 #pragma unroll
             for (int u = 0; u < NCHK * 4; ++u) { rb[u] += __shfl_xor_sync(0xffffffffu, rb[u], 8); rb[u] += __shfl_xor_sync(0xffffffffu, rb[u], 16); }
             if (pq == 0) {
@@ -361,7 +269,7 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                     *reinterpret_cast<float4*>(sRbs + g * 128 + CHK * c + 4 * ql) = make_float4(rb[4 * c], rb[4 * c + 1], rb[4 * c + 2], rb[4 * c + 3]);
             }
             __syncwarp();
-            if (lane == 0) mbar_arrive(rbdump);
+            if (lane == 0) mbar_arrive(bar.rbdump);
 #pragma unroll
             for (int u = 0; u < NCHK * 4; ++u) rb[u] = 0.f;
             ++ndump;
@@ -379,25 +287,21 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
         // (always) and, when the tile's taps fit, the F2 window chunk.  Tile coordinates come from the geometry warps (sTile).
         auto issue_chunk = [&](int q) {
             const int jt = q / NCHK, c = q - jt * NCHK, buf = q % NWB;
-            mbar_wait_parked(&recs[jt % NREC], (jt / NREC) & 1);
+            mbar_wait_parked(&bar.recs[jt % NREC], (jt / NREC) & 1);
             const int* ti = sTile + (jt % NREC) * 8;
             const int b = ti[0], tx0 = ti[1], ty0 = ti[2];
             int wx0, wy0;
-#ifdef BANET_TC7_DBG_NOTMA          // timing experiment only: nothing is loaded (results are garbage)
-            mbar_arrive(&winfull[buf]); (void)b; (void)tx0; (void)ty0; (void)wx0; (void)wy0; (void)c;
-#else
             const bool staged = decide(jt, wx0, wy0);
             unsigned char* dst = base + SM::off_win + buf * WBUF;
-            mbar_arrive_expect_tx(&winfull[buf], (staged ? WIN_TX_BYTES : 0) + C1_BYTES);
+            mbar_arrive_expect_tx(&winfull[buf], (staged ? WIN_BYTES : 0) + C1_BYTES);
             tma_load_4d(dst + WIN_BYTES, &tmapC, c * CHK, tx0, ty0, b, &winfull[buf]);
             if (staged) tma_load_4d(dst, &tmapF, c * CHK, wx0, wy0, b, &winfull[buf]);
-#endif
         };
         if (g == 0) { if (lane == 0) { for (int q = 0; q < NWB && q < nchunks; ++q) issue_chunk(q); } __syncwarp(); }
 
         for (int j = 0; j < ntiles; ++j) {
             const int s = j % NREC;
-            mbar_wait_parked(&recs[s], (j / NREC) & 1);
+            mbar_wait_parked(&bar.recs[s], (j / NREC) & 1);
             const int b = sTile[s * 8];
             if (b != cur_b) { if (cur_b >= 0) dump_rb(); cur_b = b; }
             int wx0, wy0;
@@ -432,11 +336,7 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
             for (int c = 0; c < NCHK; ++c) {
                 const int q = j * NCHK + c, buf = q % NWB;
                 mbar_wait_parked(&winfull[buf], (q / NWB) & 1);
-#ifdef BANET_TC7_DBG_NOGATHER       // timing experiment only: no tap loads / arithmetic (results are garbage)
-                if (false) {
-#else
                 if (mask != 0.f) {
-#endif
                     // grad_fixed on the fly (bundlenet.py:92-100): 2gx, 2gy = central differences at the 4 bilinear taps, as sums of positive minus sums of
                     // negative terms in packed fp32 pairs; the factors 1/2 are applied once per pixel.  Two load phases (the two middle rows, then the rows
                     // above / below) keep at most 8 of the 12 taps live; the empty asm ties phase B's address to a phase-A result so that ptxas cannot hoist it.
@@ -516,10 +416,10 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
             // ---- scaling pass: R row = rna(s_n * b_n) (the MMA's B operand), and the A-operand side of the precision mode, for this quarter's pixel:
             //      16 floats per lane = its 16-B chunk in each of the 4 basis blocks (a quarter reads / writes one whole 128-B row: conflict-free).
             //      Moved here from the 4 algebra warps: 16 warps share the work and the algebra -> MMA path of a tile becomes short.
-            if (j > 0) mbar_wait_parked(rfree, (j - 1) & 1);                  // MMAs of tile j-1 done: R (and A_lo) are free
+            if (j > 0) mbar_wait_parked(bar.rfree, (j - 1) & 1);              // MMAs of tile j-1 done: R (and A_lo) are free
             {
                 const int st = j % NST;
-                mbar_wait_parked(&fullB[st], (j / NST) & 1);                  // long complete (the geometry warps needed it)
+                mbar_wait_parked(&bar.fullB[st], (j / NST) & 1);              // long complete (the geometry warps needed it)
                 unsigned char* As = base + SM::off_A + st * STAGE_A;
                 unsigned char* Rs = base + SM::off_R;
                 const uint32_t rowo = sw128_32b_off(pxi, ql);
@@ -530,25 +430,15 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                     const uint32_t off = blk * 8192 + rowo;
                     const float4 bv = *reinterpret_cast<const float4*>(As + off);
                     *reinterpret_cast<float4*>(Rs + off) = make_float4(tf32_rna_bits(sn * bv.x), tf32_rna_bits(sn * bv.y), tf32_rna_bits(sn * bv.z), tf32_rna_bits(sn * bv.w));
-                    if constexpr (MODE == 1) {
-                        // single-pass mode: the basis tile is rounded to tf32 IN PLACE with a dither hashed from (iterate, pixel, column): unbiased, changes
-                        // with the iterate, and a pure function of the inputs (see generation 6 for the measurements that led here)
-                        uint32_t hsh = hbase ^ ((uint32_t)(blk * 8 + ql) * 0x85EBCA77u);
-                        hsh ^= hsh >> 16; hsh *= 0x7FEB352Du; hsh ^= hsh >> 15;
-                        uint32_t hs2 = hsh * 0x846CA68Bu; hs2 ^= hs2 >> 16;
-                        *reinterpret_cast<float4*>(As + off) =
-                            make_float4(__uint_as_float((__float_as_uint(bv.x) + (hsh & 0x1fffu)) & 0xFFFFE000u),
-                                        __uint_as_float((__float_as_uint(bv.y) + ((hsh >> 13) & 0x1fffu)) & 0xFFFFE000u),
-                                        __uint_as_float((__float_as_uint(bv.z) + (hs2 & 0x1fffu)) & 0xFFFFE000u),
-                                        __uint_as_float((__float_as_uint(bv.w) + ((hs2 >> 13) & 0x1fffu)) & 0xFFFFE000u));
-                    }
+                    if constexpr (MODE == 1)     // single-pass mode: the basis tile is rounded to tf32 IN PLACE
+                        *reinterpret_cast<float4*>(As + off) = tf32_stochastic4(bv, hbase ^ ((uint32_t)(blk * 8 + ql) * 0x85EBCA77u));
                     if constexpr (MODE >= 2)
                         *reinterpret_cast<float4*>(base + SM::off_Alo + off) = make_float4(bv.x - tf32_trunc(bv.x), bv.y - tf32_trunc(bv.y), bv.z - tf32_trunc(bv.z), bv.w - tf32_trunc(bv.w));
                 }
             }
             fence_proxy_async_smem();                        // the MMA reads R / A / A_lo through the async proxy
             __syncwarp();
-            if (lane == 0) mbar_arrive(&gath[s]);
+            if (lane == 0) mbar_arrive(&bar.gath[s]);
         }
         if (cur_b >= 0) dump_rb();
     } else if (warp < W0 + GW + AW) {
@@ -557,7 +447,6 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
         const int awi = warp - (W0 + GW);                    // 0..3: pixels / rows 16*awi .. 16*awi+15
         const int atid = tid - (W0 + GW) * 32;
         const int nlr = awi * 16 + r16;
-        const SlotLayout L{KR, C};
         unsigned char* Rs = base + SM::off_R;
         float cc[28];
 #pragma unroll
@@ -573,42 +462,12 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
 
         auto issue_tma = [&](int t) {                        // basis tile t -> stage t % NST (elected thread)
             const int st = t % NST;
-            const TileCoord tc = tile_coord(prm, t_begin + t);
-            mbar_arrive_expect_tx(&fullB[st], KBLK * 8192);
+            const TileCoord tc = banded_tile_coord(prm, t_begin + t);
+            mbar_arrive_expect_tx(&bar.fullB[st], KBLK * 8192);
             unsigned char* dst = base + SM::off_A + st * STAGE_A;
-            if (grid2d) {
 #pragma unroll
-                for (int blk = 0; blk < KBLK; ++blk) tma_load_3d(dst + blk * 8192, &tmapB, blk * 32, tc.tx0, tc.b * prm.grid_h + tc.ty0, &fullB[st]);
-            } else {
-                const int row = tc.b * N + tc.n0;
-#pragma unroll
-                for (int blk = 0; blk < KBLK; ++blk) tma_load_2d(dst + blk * 8192, &tmapB, blk * 32, row, &fullB[st]);
-            }
+            for (int blk = 0; blk < KBLK; ++blk) tma_load_3d(dst + blk * 8192, &tmapB, blk * 32, tc.tx0, tc.b * prm.grid_h + tc.ty0, &bar.fullB[st]);
         };
-        auto flush = [&](int sp) {
-            float* slot = prm.partials + ((size_t)blockIdx.x * prm.max_span + sp) * prm.slot_floats;
-            // H_cc / g_c / nvalid: 16 pixel-lanes -> warp total (fixed shuffle tree) -> 4 warp partials summed in fixed order
-#pragma unroll
-            for (int q = 0; q < 28; ++q) {
-                float v = cc[q];
-                v += __shfl_xor_sync(0xffffffffu, v, 8); v += __shfl_xor_sync(0xffffffffu, v, 4);
-                v += __shfl_xor_sync(0xffffffffu, v, 2); v += __shfl_xor_sync(0xffffffffu, v, 1);
-                if (lane == 0) sCcs[awi * 28 + q] = v;
-                cc[q] = 0.f;
-            }
-            mbar_wait_parked(rbdump, sp & 1);                // the gather warps parked their |diff| sums for this pair
-            team_bar<AW * 32>();
-            if (atid < C) {
-                float sum = 0.f;
-#pragma unroll
-                for (int wq = 0; wq < GW; ++wq) sum += sRbs[wq * 128 + atid];
-                slot[L.off_rbar() + atid] = sum;
-            }
-            if (atid < 28) slot[L.off_cc() + atid] = (sCcs[atid] + sCcs[28 + atid]) + (sCcs[56 + atid] + sCcs[84 + atid]);
-            team_bar<AW * 32>();
-            if (lane == 0) mbar_arrive(rbfree);
-        };
-
         if (awi == 0 && lane == 0)
             for (int t = 0; t < NST && t < ntiles; ++t) issue_tma(t);      // every stage starts free
 
@@ -620,68 +479,32 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                 // MMAs of tile j-1 done: R / A_lo and stage (j-1) % NST are free.  Refill the stage BEFORE waiting for the gather of tile j: the
                 // window producer (gather warp 0) looks ahead into tile j+1 and waits for its records, i.e. for the geometry warps, i.e. for
                 // this very TMA when NST == 2 -- issued after gath[j] it would close a cycle through the gather warps themselves.
-                mbar_wait_parked(rfree, (j - 1) & 1);
+                mbar_wait_parked(bar.rfree, (j - 1) & 1);
                 if (awi == 0 && lane == 0 && j - 1 + NST < ntiles) issue_tma(j - 1 + NST);
             }
-            mbar_wait_parked(&gath[sr], (j / NREC) & 1);
+            mbar_wait_parked(&bar.gath[sr], (j / NREC) & 1);
             const int b = sTile[sr * 8];
             if (b != scale_b) { scale_b = b; ++sspan; fx = __ldg(prm.intr + b * 4); fy = __ldg(prm.intr + b * 4 + 1); }
             float ext[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-            if (lane < 16) {                                 // thread per pixel (bundlenet.py:49-74)
-                const float* rec = sRec + (sr * TILE + nlr) * REC;
-                const float4 ra = *reinterpret_cast<const float4*>(rec + 12), rbq = *reinterpret_cast<const float4*>(rec + 4),
-                             rc = *reinterpret_cast<const float4*>(rec + 8);
-                if (rbq.x != 0.f) {
-                    const float m11 = ra.x, m12 = ra.y, m22 = ra.z, q1 = ra.w, q2 = rc.w, x = rbq.y, y = rbq.z, iZ = rbq.w;
-                    const float rx = rc.x, ry = rc.y, rz = rc.z;
-                    const float a0[6] = {-fx * (x * y), -fx * (-1.f - x * x), -fx * y, -fx * (-iZ), 0.f, -fx * (x * iZ)};
-                    const float a1[6] = {-fy * (1.f + y * y), -fy * (-(x * y)), -fy * (-x), 0.f, -fy * (-iZ), -fy * (y * iZ)};
-                    float ux[6], uy[6];
-#pragma unroll
-                    for (int i = 0; i < 6; ++i) { ux[i] = m11 * a0[i] + m12 * a1[i]; uy[i] = m12 * a0[i] + m22 * a1[i]; }
-                    int q = 0;
-#pragma unroll
-                    for (int i = 0; i < 6; ++i)
-#pragma unroll
-                        for (int jj = i; jj < 6; ++jj) { cc[q] += a0[i] * ux[jj] + a1[i] * uy[jj]; ++q; }
-#pragma unroll
-                    for (int i = 0; i < 6; ++i) cc[21 + i] += a0[i] * q1 + a1[i] * q2;
-                    cc[27] += 1.f;
-                    const float jd0 = fx * ((rx - rz * x) * iZ), jd1 = fy * ((ry - rz * y) * iZ);
-                    const float u0 = m11 * jd0 + m12 * jd1, u1 = m12 * jd0 + m22 * jd1;
-#pragma unroll
-                    for (int i = 0; i < 6; ++i) ext[i] = a0[i] * u0 + a1[i] * u1;
-                    ext[6] = jd0 * q1 + jd1 * q2;
-                    ext[7] = jd0 * u0 + jd1 * u1;
-                }
-            }
+            if (lane < 16) pixel_algebra(sRec + (sr * TILE + nlr) * REC, fx, fy, cc, ext);
             __syncwarp();
-            if (lane == 0) mbar_arrive(&recfree[sr]);        // the record buffer may be refilled (everything needed is in registers)
-            mbar_wait_parked(&fullB[s], (j / NST) & 1);      // long complete; orders the TMA writes before the reads below
-            if (lane < 16) {                                 // R columns 128..134 = [v(6) | t], column 135 stays zero
-                const float4 e0 = make_float4(tf32_rna(ext[0]), tf32_rna(ext[1]), tf32_rna(ext[2]), tf32_rna(ext[3]));
-                const float4 e1 = make_float4(tf32_rna(ext[4]), tf32_rna(ext[5]), tf32_rna(ext[6]), 0.f);
-                *reinterpret_cast<float4*>(Rs + EXTB * 8192 + sw128_32b_off(nlr, 0)) = e0;
-                *reinterpret_cast<float4*>(Rs + EXTB * 8192 + sw128_32b_off(nlr, 1)) = e1;
-                if constexpr (MODE == 3) {
-                    *reinterpret_cast<float4*>(base + SM::off_Rlo + EXTB * 8192 + sw128_32b_off(nlr, 0)) = make_float4(ext[0] - e0.x, ext[1] - e0.y, ext[2] - e0.z, ext[3] - e0.w);
-                    *reinterpret_cast<float4*>(base + SM::off_Rlo + EXTB * 8192 + sw128_32b_off(nlr, 1)) = make_float4(ext[4] - e1.x, ext[5] - e1.y, ext[6] - e1.z, 0.f);
-                }
-            }
+            if (lane == 0) mbar_arrive(&bar.recfree[sr]);    // the record buffer may be refilled (everything needed is in registers)
+            mbar_wait_parked(&bar.fullB[s], (j / NST) & 1);  // long complete; orders the TMA writes before the reads below
+            if (lane < 16) write_vt<MODE, KBLK>(Rs, nullptr, nlr, ext);
             // (the R rows s_n * b_n were written by the gather warps' scaling pass; this team only adds the [v | t] block)
             fence_proxy_async_smem();
             team_bar<AW * 32>();                           // all 64 rows written
             if (awi == 0) {
                 if (lane == 0) {                             // ---- tcgen05.mma issue for this tile
-                    if (new_span) { mbar_wait_parked(tmemfree, (mspan & 1) ^ 1); accL = 0; new_span = false; }
-                    if (tic == 0) { ++chain; set = chain & 1; mbar_wait_parked(&drained[set], ((chain >> 1) & 1) ^ 1); accH = 0; }
+                    if (new_span) { mbar_wait_parked(bar.tmemfree, (mspan & 1) ^ 1); accL = 0; new_span = false; }
+                    if (tic == 0) { ++chain; set = chain & 1; mbar_wait_parked(&bar.drained[set], ((chain >> 1) & 1) ^ 1); accH = 0; }
                     tc_fence_after_sync();
                     const uint32_t ahi = smem_u32(base + SM::off_A + s * STAGE_A);
-                    const uint32_t rhi = smem_u32(base + SM::off_R), rlo = smem_u32(base + SM::off_Rlo), alo = smem_u32(base + SM::off_Alo);
+                    const uint32_t rhi = smem_u32(base + SM::off_R), alo = smem_u32(base + SM::off_Alo);
 #pragma unroll
-                    for (int pass = 0; pass < MODE; ++pass) {
+                    for (int pass = 0; pass < MODE; ++pass) {     // no R_lo pass: MODE <= 2
                         const uint32_t a0 = (pass == 1) ? alo : ahi;
-                        const uint32_t r0 = (pass == 2) ? rlo : rhi;
+                        const uint32_t r0 = rhi;
                         const uint32_t dcol = tmem + (pass == 0 ? set * NN : ACCL);
 #pragma unroll
                         for (int kk = 0; kk < TILE / 8; ++kk) {
@@ -690,91 +513,18 @@ lm_build_tc7_kernel(const __grid_constant__ CUtensorMap tmapB, const __grid_cons
                             if (pass == 0) accH = 1; else accL = 1;
                         }
                     }
-                    mma_commit(rfree);
-                    if (++tic == CHAIN) { mma_commit(&chain_done[set]); tic = 0; }
-                    if (last_of_pair) { if (tic > 0) mma_commit(&chain_done[set]); mma_commit(flushb); ++mspan; tic = 0; new_span = true; }
+                    mma_commit(bar.rfree);
+                    if (++tic == CHAIN) { mma_commit(&bar.chain_done[set]); tic = 0; }
+                    if (last_of_pair) { if (tic > 0) mma_commit(&bar.chain_done[set]); mma_commit(bar.flushb); ++mspan; tic = 0; new_span = true; }
                 }
                 __syncwarp();
             }
-            if (last_of_pair) flush(sspan);
+            if (last_of_pair) flush<KBLK, C>(prm, bar, cc, sspan, sCcs, sRbs, awi, atid, lane);
         }
     } else {
-        // ===================================================================== drainer warps: TMEM -> partial slots, fully asynchronous
-        setmaxnreg_dec<40>();
-        const int dq = warp - (W0 + GW + AW);                // TMEM lane quadrant (= warp % 4)
-        const SlotLayout L{KR, C};
-        const uint64_t pol_slot = l2_policy_evict_last();    // keep the CTA's partial slot L2-resident between two chains (see lm_build_tc6.cu)
-        auto drain_region = [&](float* slot, uint32_t col0, bool overwrite) {
-            const int row = dq * 32 + lane;
-            if (KBLK != 4 && dq * 32 >= KR) return;          // this lane quadrant holds no basis row (warp-uniform)
-            const uint32_t tq = tmem + ((uint32_t)(dq * 32) << 16) + col0;
-            float v[16];
-#pragma unroll 1
-            for (int cb = 0; cb < KR / 16; ++cb) {
-                tmem_ld_32x16(tq + cb * 16, v);
-                float* dst = slot + (size_t)(cb * 16) * KR + row;
-                if (overwrite) {
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) st_f32_hint(dst + (size_t)j * KR, v[j], pol_slot);
-                } else {
-#pragma unroll
-                    for (int hb = 0; hb < 16; hb += 8) {
-                        float o[8];
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) o[j] = ld_f32_hint(dst + (size_t)(hb + j) * KR, pol_slot);
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) st_f32_hint(dst + (size_t)(hb + j) * KR, o[j] + v[hb + j], pol_slot);
-                    }
-                }
-            }
-            tmem_ld_32x16(tq + KR, v);
-            float* dst = slot + L.off_ext() + row;
-#pragma unroll
-            for (int r = 0; r < 7; ++r) {
-                if (overwrite) st_f32_hint(dst + r * KR, v[r], pol_slot);
-                else st_f32_hint(dst + r * KR, ld_f32_hint(dst + r * KR, pol_slot) + v[r], pol_slot);
-            }
-        };
-        int chain = -1, tic = 0, span = 0, cur_b = -1;
-        bool first = true;
-        int b = (ntiles > 0) ? (int)((unsigned)t_begin / (unsigned)prm.tiles_per_pair) : 0;
-        int rr = (ntiles > 0) ? (int)((unsigned)t_begin - (unsigned)b * (unsigned)prm.tiles_per_pair) : 0;
-        auto drain_hi = [&]() {
-            const int set = chain & 1;
-            float* slot = prm.partials + ((size_t)blockIdx.x * prm.max_span + span) * prm.slot_floats;
-            mbar_wait_parked(&chain_done[set], (chain >> 1) & 1);
-            tc_fence_after_sync();
-            drain_region(slot, set * NN, first);
-            first = false;
-            tc_fence_before_sync();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&drained[set]);
-        };
-        auto end_span = [&]() {
-            if (tic > 0) drain_hi();
-            if constexpr (MODE >= 2) {
-                float* slot = prm.partials + ((size_t)blockIdx.x * prm.max_span + span) * prm.slot_floats;
-                mbar_wait_parked(flushb, span & 1);
-                tc_fence_after_sync();
-                drain_region(slot, ACCL, false);
-                tc_fence_before_sync();
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(tmemfree);
-            ++span;
-        };
-        for (int it = 0; it < ntiles; ++it) {
-            if (b != cur_b) { if (cur_b >= 0) end_span(); cur_b = b; tic = 0; first = true; }
-            if (tic == 0) ++chain;
-            if (++tic == CHAIN) { drain_hi(); tic = 0; }
-            if (++rr == prm.tiles_per_pair) { rr = 0; ++b; }
-        }
-        if (cur_b >= 0) end_span();
+        drainer_role<40, MODE, KBLK, C>(prm, bar, tmem, t_begin, ntiles, warp - (W0 + GW + AW), lane);
     }
-
-    tc_fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TMEM_COLS>(tmem);
+    release_tmem(tmem, warp);
 }
 
 
@@ -793,7 +543,7 @@ static int launch7(const CUtensorMap& tmB, const CUtensorMap& tmF, const CUtenso
 }  // namespace v7
 
 bool lm_build_tc7_supported(int mode, int nch, int kblk) { return (mode == 1 || mode == 2) && (nch == 1 || nch == 2) && kblk == 4; }
-void lm_build_tc7_window(int* wx, int* wy) { *wx = v7::WX; *wy = v7::BOX_Y; }
+void lm_build_tc7_window(int* wx, int* wy) { *wx = v7::WX; *wy = v7::WY; }
 
 int lm_build_tc7_launch(int mode, int nch, int kblk, const CUtensorMap& tmB, const CUtensorMap& tmF, const CUtensorMap& tmC, const BuildParams& prm, int grid,
                         cudaStream_t st)

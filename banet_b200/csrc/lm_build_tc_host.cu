@@ -104,7 +104,6 @@ int lm_build_tc(const banet_level_t* lv, const BuildPlan& plan, int mode, const 
     prm.band_rows = 1; prm.l2_hints = 0; prm.tap_prefetch = 0; prm.kq_i = 0; prm.kq_j = 0;
     prm.hdd_transposed = 1;
     prm.force_direct = g_tuning.tc7_force_direct;
-    prm.trace = nullptr;
     const int nch = lv->C / 64;
     if (use_gen7(lv, mode, kblk)) {
         int band = g_tuning.tc7_band_rows; if (band < 1) band = 1; if (band > prm.tiles_y) band = prm.tiles_y;

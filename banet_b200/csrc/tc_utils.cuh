@@ -39,14 +39,6 @@ __device__ __forceinline__ void mbar_wait_parked(uint64_t* bar, uint32_t parity)
     asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n\t@p bra DONE_%=;\n\tbra WAIT_%=;\n\tDONE_%=:\n\t}"
                  :: "r"(smem_u32(bar)), "r"(parity), "r"(0x989680) : "memory");
 }
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity) {      // for single-thread role warps: back off
-    while (!mbar_try_wait(bar, parity)) { __nanosleep(40); }
-}
-// best-effort wait (for the prefetcher, which must never hang the CTA): gives up after ~max_iters polls
-__device__ __forceinline__ bool mbar_wait_bounded(uint64_t* bar, uint32_t parity, int max_iters) {
-    for (int i = 0; i < max_iters; ++i) { if (mbar_try_wait(bar, parity)) return true; __nanosleep(64); }
-    return false;
-}
 template <int NREG> __device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" :: "n"(NREG)); }
 template <int NREG> __device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" :: "n"(NREG)); }
 
@@ -103,14 +95,9 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* m, int
                  :: "r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
 
-// L2 prefetches (no destination, no completion): a contiguous range, or a tensor-map box
+// L2 prefetch of a contiguous range (no destination, no completion)
 __device__ __forceinline__ void prefetch_l2_bulk(const void* p, uint32_t bytes) {      // bytes % 16 == 0, p 16-B aligned
     asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" :: "l"(p), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void prefetch_l2_line(const void* p) { asm volatile("prefetch.global.L2 [%0];" :: "l"(p)); }
-__device__ __forceinline__ void prefetch_l2_tensor_4d(const CUtensorMap* m, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
-                 :: "l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
 
 // ---------------------------------------------------------------- tcgen05 / TMEM
@@ -192,7 +179,19 @@ __device__ __forceinline__ float tf32_rna(float x) {          // round to neares
 }
 // round-to-nearest (ties away) for an operand whose low 13 bits the tensor core ignores anyway: one integer add, no mask
 __device__ __forceinline__ float tf32_rna_bits(float x) { return __uint_as_float(__float_as_uint(x) + 0x1000u); }
-__device__ __forceinline__ float tf32_rna_mask(float x) { return __uint_as_float((__float_as_uint(x) + 0x1000u) & 0xFFFFE000u); }
 __device__ __forceinline__ float tf32_trunc(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
+// Stochastic rounding of 4 values to tf32 with a dither hashed from `h` (the single-pass mode's basis tile: h mixes the iterate, the pixel
+// and the column).  Truncation would bias the products (relH 1e-5); round-to-nearest is unbiased per launch (relH < 1e-6) but applies the
+// SAME perturbation to the basis at every LM iteration, so its effect adds up coherently over a solve (W off by 1e-3 after 20 iterations).
+// The dither is unbiased AND changes with the iterate, like the rounding of R does; it is a pure function of the inputs, so results stay
+// bit-reproducible.
+__device__ __forceinline__ float4 tf32_stochastic4(float4 v, uint32_t h) {
+    h ^= h >> 16; h *= 0x7FEB352Du; h ^= h >> 15;
+    uint32_t h2 = h * 0x846CA68Bu; h2 ^= h2 >> 16;
+    return make_float4(__uint_as_float((__float_as_uint(v.x) + (h & 0x1fffu)) & 0xFFFFE000u),
+                       __uint_as_float((__float_as_uint(v.y) + ((h >> 13) & 0x1fffu)) & 0xFFFFE000u),
+                       __uint_as_float((__float_as_uint(v.z) + (h2 & 0x1fffu)) & 0xFFFFE000u),
+                       __uint_as_float((__float_as_uint(v.w) + ((h2 >> 13) & 0x1fffu)) & 0xFFFFE000u));
+}
 
 }}  // namespace banet::tc

@@ -1,4 +1,4 @@
-"""CPU model of the shared-memory addressing used by the generation-6 build kernel (banet_b200/csrc/lm_build_tc6.cu):
+"""CPU model of the shared-memory addressing used by the tensor-core build kernels (banet_b200/csrc/lm_build_tc_roles.cuh, lm_build_tc6.cu):
 the 128-B swizzle with 32-B atoms (tc_utils.cuh: sw128_32b_off) and the rotated lane -> chunk walks of the b.W and R-row
 loops.  Proves on the host what the kernel relies on: coverage (every element visited exactly once) and bank-conflict
 freedom (each quarter-warp of a 128-bit access touches 8 distinct 16-B bank groups)."""
